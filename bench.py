@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py - the hot path of BASELINE.json measured on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C3|C1|C5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload C3|C1|C5] [--dump-outputs DIR]
   (N > 1: launched by torch.distributed.run, one rank per GPU, NCCL)
+
+--steps K is the number of timed calls in every timed loop (a loop with a stalled call is timed once more: see
+`remeasured` below).  --dump-outputs DIR: after the timed steps, the outputs of the
+last timed FINCH call are written as DIR/<name>.npy in float64 (see dump_outputs); the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 
 Workload (config.workload), default BASELINE configs[2]/[3]: FINCH full hierarchy on N = 240 000 x D = 512 synthetic
 Gaussian-mixture embeddings (Kinetics-400 train size), seed 0 (video_similarity_search_b200.synth).  A "step" is one
@@ -61,7 +66,11 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-nn", action="store_true", help="reference arm: skip the one full pass of the level-0 stage")
     ap.add_argument("--no-retrieval", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a sample of the work and has no step output to write")
+    return args
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum of ONE launch of the dominant kernel from a committed `ncu --set full`
@@ -219,6 +228,27 @@ while True:
 def has_stalled_call(host_ms_per_call, factor=2.5):
     """The re-measurement rule of the timed loops: one call took more than `factor` x the median call."""
     return len(host_ms_per_call) >= 3 and max(host_ms_per_call) > factor * statistics.median(host_ms_per_call)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, c, num_clust, max_bytes=DUMP_BYTES):
+    """Write what FINCH returned to its caller as float64 .npy files (labels are integers, exact in float64):
+    c.npy [N, P] and num_clust.npy [P].  When the label matrix would take the files over `max_bytes`, c.npy holds a
+    fixed sample of its rows (seed 0, ascending) and c_rows.npy their indices."""
+    os.makedirs(out_dir, exist_ok=True)
+    c = np.asarray(c)
+    arrays = {"num_clust": np.asarray(num_clust, dtype=np.float64)}
+    room = max_bytes - arrays["num_clust"].nbytes
+    if c.size * 8 <= room:
+        arrays["c"] = c.astype(np.float64)
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(c.shape[0], room // (8 * (c.shape[1] + 1)), replace=False))
+        arrays["c"] = c[rows].astype(np.float64)
+        arrays["c_rows"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -582,7 +612,7 @@ def run_b200(args):
         if not big:
             tr, _, te, _ = synth.c2_retrieval()
             retrieval["C2_top50"] = retrieval_record(torch, be, lib, peaks, be.to_device(te), be.to_device(tr), 50,
-                                                     max(args.steps, 10), world, "BASELINE configs[1], host-generated", True)
+                                                     args.steps, world, "BASELINE configs[1], host-generated", True)
         if big or (world == 1 and args.workload == "C3"):
             if big:
                 xq = x_dev
@@ -592,7 +622,7 @@ def run_b200(args):
             g = torch.Generator(device=be.device).manual_seed(1)
             q5 = cen[torch.randint(0, cen.shape[0], (C5_QUERIES,), device=be.device, generator=g)] + \
                 torch.randn(C5_QUERIES, cen.shape[1], device=be.device, generator=g)
-            retrieval["C5_top50"] = retrieval_record(torch, be, lib, peaks, q5, xq, 50, 3, world,
+            retrieval["C5_top50"] = retrieval_record(torch, be, lib, peaks, q5, xq, 50, args.steps, world,
                                                      "BASELINE configs[4] retrieval shape (Q not fixed by BASELINE: 100 000), "
                                                      "device-generated mixture", False)
             del q5
@@ -727,6 +757,8 @@ def run_b200(args):
     if sharded_equal is not None:
         parity["sharded_first_neighbors_equal_single_gpu_on_every_rank"] = sharded_equal
     line["parity"] = parity
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, c, num_clust)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

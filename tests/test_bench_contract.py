@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -46,9 +47,17 @@ def test_reference_arm_uses_all_cores_under_torchrun_environment():
 
 
 @pytest.mark.gpu
-def test_b200_arm_prints_the_contract_line():
-    line = _run(["--workload", "C1", "--steps", "2", "--warmup", "3", "--cpu-sample-rows", "512"])
+def test_b200_arm_prints_the_contract_line(tmp_path, golden_dir):
+    line = _run(["--workload", "C1", "--steps", "2", "--warmup", "3", "--cpu-sample-rows", "512",
+                 "--dump-outputs", str(tmp_path)])
     assert BASE_KEYS <= set(line) and "impl" not in line
+    assert len(line["step_host_ms_rank0"]) == 2
+    # the outputs of the last timed call: the label matrix of the unmodified reference on every row but ties (C1 has one)
+    c, num_clust = np.load(tmp_path / "c.npy"), np.load(tmp_path / "num_clust.npy")
+    assert c.dtype == num_clust.dtype == np.float64 and not (tmp_path / "c_rows.npy").exists()
+    g = np.load(os.path.join(golden_dir, "c1_9537x512.npz"))
+    assert num_clust.tolist() == [1170, 101, 25, 8, 5] and c.shape == (9537, 5)
+    assert (c != g["c"]).any(axis=1).sum() <= 2
     assert {"gpu_launches", "clocks", "roofline", "nn_stage", "finch_seconds", "parity", "e2e_pageable", "retrieval"} <= set(line)
     assert line["gpu_launches"] > 0 and line["n_gpus"] == 1 and line["steps"] == 2 and line["warmup"] >= 3
     rf = line["roofline"]
@@ -67,6 +76,21 @@ def test_b200_arm_prints_the_contract_line():
     assert line["retrieval"]["C2_top50"]["indices_equal_exact_kernels"] is True
     cb = line["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["unit"] == line["unit"]
+
+
+def test_dumped_outputs_stay_within_their_budget(tmp_path):
+    """bench.dump_outputs: a label matrix too large for the budget is written as the same seeded row sample every time."""
+    import bench
+    c = np.arange(3000 * 4, dtype=np.int32).reshape(3000, 4)
+    bench.dump_outputs(tmp_path / "full", c, [3000, 40, 5, 2])
+    assert np.array_equal(np.load(tmp_path / "full" / "c.npy"), c) and not (tmp_path / "full" / "c_rows.npy").exists()
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, c, [3000, 40, 5, 2], max_bytes=20000)
+        assert sum(f.stat().st_size for f in (tmp_path / run).iterdir()) <= 20000 + 3 * 128      # (+ .npy headers)
+    rows = np.load(tmp_path / "a" / "c_rows.npy")
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "c_rows.npy")) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "c.npy"), c[rows.astype(np.int64)])
+    assert np.load(tmp_path / "a" / "num_clust.npy").tolist() == [3000, 40, 5, 2]
 
 
 def test_stall_rule_of_the_timed_loops():

@@ -1,14 +1,11 @@
 """The oracle (oracle/finch_oracle.py) against the fixtures produced by the UNMODIFIED reference
-(tests/golden/make_golden.py) and, when /root/reference is present, against the live reference."""
-import contextlib
-import io
+(tests/golden/make_golden.py)."""
 import os
 
 import numpy as np
 import pytest
 
 from oracle import finch_oracle as fo
-from oracle import reference_harness as rh
 from tests.golden.make_golden import CASES, make_input
 
 SMALL = [k for k in CASES if k != "c1_9537x512"]
@@ -94,21 +91,18 @@ def test_cluster_means_is_fp64_segmented_mean():
     np.testing.assert_allclose(m, direct, rtol=0, atol=1e-12)
 
 
-@pytest.mark.skipif(not rh.reference_available(), reason="/root/reference not mounted (GPU box)")
 @pytest.mark.parametrize("name", ["gmm_1200x64", "gmm_2500x96_flann"])
-def test_oracle_matches_live_reference(name):
-    case = CASES[name]
+def test_oracle_plain_call_matches_stored_reference_output(golden_dir, name):
+    """The oracle called the way a caller of the reference calls FINCH (defaults, no trace) against the partition the
+    reference computed with the same defaults (stored by make_golden.py), the second case through the FLANN branch."""
+    case, g = CASES[name], _load(golden_dir, name)
     x = make_input(case)
     thr = case.get("flann_threshold")
-    mod = rh.load_reference_finch(with_exact_flann=thr is not None)
     saved = fo.FLANN_THRESHOLD
     try:
         if thr is not None:
-            mod.FLANN_THRESHOLD = thr
             fo.FLANN_THRESHOLD = thr
-        with contextlib.redirect_stdout(io.StringIO()):
-            c_ref, n_ref, _ = mod.FINCH(x, verbose=False)
         c, n, _ = fo.finch(x)
     finally:
         fo.FLANN_THRESHOLD = saved
-    assert n == n_ref and np.array_equal(c, c_ref)
+    assert n == g["num_clust"].tolist() and np.array_equal(c, g["c"])
