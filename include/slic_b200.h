@@ -247,6 +247,31 @@ int slic_merge_cluster_sums(const double* sums_prev_dev, const int32_t* counts_p
                             double* sums_out_dev, int32_t* counts_out_dev, double* means_out_dev,
                             slic_stream_t stream);
 
+/* ---- K6: spherical k-means (clustering/cluster_masks.py fit_cluster, method='spherical_kmeans') ----------- */
+/* spherecluster SphericalKMeans(...).fit(X) over scikit-learn 0.22 helpers; the algorithm is restated in
+ * oracle/kmeans_oracle.py.  The random draws come from the caller, so that a binding reproduces any RNG's sequence.
+ *
+ * k-means++ seeding (_k_init) of the unit rows unit_dev [n, d] float32: first_id is the first seed, uniforms_host
+ * [(k - 1) * L] the L draws of each later step in order (L = 2 + int(log(k)) in the reference, 1 <= L <= 32).  Every
+ * step reads the rows once for all L candidates; sqdist(a, b) = max(|a|^2 + |b|^2 - 2 a.b, 0) in float64, rounded to
+ * float32; potentials in float64, fixed order.  seeds_out_dev [k] int32 (row indices). */
+int slic_kmeans_plusplus(const float* unit_dev, int64_t n, int32_t d, int32_t k, int64_t first_id,
+                         const double* uniforms_host, int32_t L, int32_t* seeds_out_dev, slic_stream_t stream);
+/* The whole fit of the raw rows x_dev [n, d] float32 (rows are L2-normalised first): n_init runs of seeding, Lloyd
+ * (at most max_iter iterations, stop when the float64 centre shift <= mean(var(unit, axis=0)) * tol) and the final
+ * E-step; the run with the smallest inertia is kept.  init_dev [k, d] float32 (optional, normalised before use; needs
+ * n_init == 1) replaces the seeding; otherwise first_ids_host [n_init] and uniforms_host [n_init, (k - 1) * L] are
+ * the draws of each run.  Outputs: labels_out_dev [n] int32, centers_out_dev [k, d] float32 (unit rows),
+ * *inertia_out_host, *n_iter_out_host, stats_out_host [4] int64 (optional): candidates the screen re-ranked, rows
+ * its exact finisher settled, candidate-list compactions, assignments run on the screen - summed over iterations.
+ * Refuses n < k, k < 1, n_init < 1, max_iter < 1 with SLIC_ERR_INVALID_ARG before any device work.  Blocks until the
+ * outputs are in place (one status read-back per few iterations). */
+int slic_spherical_kmeans(const float* x_dev, int64_t n, int32_t d, int32_t k, const float* init_dev,
+                          const int64_t* first_ids_host, const double* uniforms_host, int32_t L, int32_t n_init,
+                          int32_t max_iter, double tol, int32_t* labels_out_dev, float* centers_out_dev,
+                          double* inertia_out_host, int32_t* n_iter_out_host, int64_t* stats_out_host,
+                          slic_stream_t stream);
+
 /* ---- K4: label-equality masks and grouping ------------------------------------------------ */
 /* models/infoNCE.py:281-283, loss/triplet_loss.py:136-142,254-261,291-297:
  * out[i, prepend + j] = (a[i] == b[j]) ^ negate as one byte per entry (torch.bool layout),

@@ -64,6 +64,9 @@ SIGNATURES = {
     "slic_comm_finch": [_ptr, _ptr, _i64, _i32, _i32, _i32, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr],
     "slic_finch": [_ptr, _i64, _i32, _ptr, _ptr, _ptr, _i32, _i32, _i32, _ptr, _ptr, _ptr, _ptr, _ptr, _ptr],
     "slic_finch_host": [_ptr, _i64, _i32, _ptr, _i32, _i32, _ptr, _ptr, _ptr, _ptr, _ptr],
+    "slic_kmeans_plusplus": [_ptr, _i64, _i32, _i32, _i64, _ptr, _i32, _ptr, _ptr],
+    "slic_spherical_kmeans": [_ptr, _i64, _i32, _i32, _ptr, _ptr, _ptr, _i32, _i32, _i32, _f64, _ptr, _ptr, _ptr, _ptr,
+                              _ptr, _ptr],
 }
 _RESTYPES = {"slic_last_error": _c.c_char_p, "slic_launch_count": _c.c_int64}
 

@@ -431,6 +431,38 @@ class CudaBackend:
                   _p(counts), _p(means), self._stream())
         return sums, counts, means
 
+    # -- K6 spherical k-means (csrc/skmeans.cu) -------------------------------------------------------
+    def kmeans_plusplus(self, unit, k, first_id, uniforms, n_local_trials):
+        """k-means++ seeds of the float32 unit rows (slic_kmeans_plusplus).  uniforms: float64 [(k - 1) * L] host draws.
+        -> int32 device tensor [k] of row indices."""
+        n, d = unit.shape
+        u = np.ascontiguousarray(uniforms, dtype=np.float64).reshape(-1)
+        if u.size != (k - 1) * n_local_trials:
+            raise ValueError("kmeans_plusplus: need (k - 1) * L uniforms")
+        seeds = torch.empty(k, dtype=torch.int32, device=unit.device)
+        _lib.call("slic_kmeans_plusplus", _p(unit), n, d, int(k), int(first_id), u.ctypes.data if u.size else None,
+                  int(n_local_trials), _p(seeds), self._stream())
+        return seeds
+
+    def spherical_kmeans(self, x, k, init=None, first_ids=None, uniforms=None, n_local_trials=1, n_init=1, max_iter=300,
+                         tol=1e-4):
+        """The whole fit on the device (slic_spherical_kmeans).  x: float32 device [n, d] (raw rows); init: float32 device
+        [k, d] or None; first_ids int64 [n_init] and uniforms float64 [n_init, (k - 1) * L]: the host draws.
+        -> (labels int32 [n], centres float32 [k, d] (device tensors), inertia float, n_iter int, stats int64 [4])."""
+        n, d = x.shape
+        labels = torch.empty(n, dtype=torch.int32, device=x.device)
+        centres = torch.empty((k, d), dtype=torch.float32, device=x.device)
+        inertia, n_iter = ctypes.c_double(0.0), ctypes.c_int32(0)
+        stats = np.zeros(4, dtype=np.int64)
+        fid = None if first_ids is None else np.ascontiguousarray(first_ids, dtype=np.int64)
+        u = None if uniforms is None else np.ascontiguousarray(uniforms, dtype=np.float64)
+        with torch.cuda.device(self.device):
+            _lib.call("slic_spherical_kmeans", _p(x), n, d, int(k), _p(init), None if fid is None else fid.ctypes.data,
+                      None if u is None or u.size == 0 else u.ctypes.data, int(n_local_trials), int(n_init), int(max_iter),
+                      float(tol), _p(labels), _p(centres), ctypes.addressof(inertia), ctypes.addressof(n_iter),
+                      stats.ctypes.data, self._stream())
+        return labels, centres, inertia.value, n_iter.value, stats
+
     # -- whole hierarchy (csrc/finch_driver.cu) ------------------------------------------------------
     FINCH_CAPACITY = 32   # label columns provided to the native driver (a FINCH level at least halves the clusters
                           # unless the min_sim cut intervenes; more levels -> SlicError status -5, see FINCH())

@@ -15,7 +15,7 @@ OBJ_DIR = os.path.join(CSRC, "build")
 LIB_PATH = os.path.join(PKG_DIR, "libslic_b200.so")
 
 SOURCES = ["api.cu", "primitives.cu", "prep.cu", "nn_exact.cu", "nn_screen_tc.cu", "cc.cu", "segmean.cu", "finch_small.cu",
-           "masks.cu", "metrics.cu", "host_entry.cu", "finch_driver.cu", "comm.cu"]
+           "masks.cu", "metrics.cu", "host_entry.cu", "finch_driver.cu", "comm.cu", "skmeans.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

@@ -14,19 +14,28 @@ import torch
 
 from .. import backend as _backend
 from .finch import FINCH
+from .spherical_kmeans import SphericalKMeans
 
 _METHODS = ['DBSCAN', 'Agglomerative', 'OPTICS', 'kmeans', 'spherical_kmeans', 'finch']
 
 
 def fit_cluster(embeddings, method='Agglomerative', k=1000, l2normalize=True, finch_partition=0):
-    """cluster_masks.py:38-98.  Only method='finch' (the one the shipped configs use,
-    config/custom_configs/resnet_ucf_itercluster_flow.yaml:49-50) runs on the B200 path; the sklearn /
-    spherecluster methods are outside the hot path and raise NotImplementedError.
+    """cluster_masks.py:38-98.  method='finch' (the one the shipped configs use,
+    config/custom_configs/resnet_ucf_itercluster_flow.yaml:49-50) and method='spherical_kmeans'
+    (SphericalKMeans(n_clusters=k), clustering/spherical_kmeans.py) run on the B200 path; the sklearn methods
+    are outside it and raise NotImplementedError.  l2normalize has no effect on spherical_kmeans, which
+    normalises the rows itself.
 
     embeddings: torch tensor [N, D] (CPU as the reference passes it, or already on the GPU - then the
     host round trip of cluster_masks.py:80 is skipped).  Returns int32 labels [N] (numpy)."""
     assert(method in _METHODS)                                       # cluster_masks.py:42-43
     print("Clustering with {}...".format(method))
+    if method == 'spherical_kmeans':
+        if isinstance(embeddings, torch.Tensor):
+            embeddings = embeddings.detach()
+        labels = SphericalKMeans(n_clusters=k).fit(embeddings).labels_
+        print("Fitted " + str(k) + " clusters with " + str(method))
+        return labels
     if method != 'finch':
         raise NotImplementedError("method=%r is not on the B200 hot path; use the reference for it" % method)
     if isinstance(embeddings, torch.Tensor):
