@@ -146,11 +146,11 @@ int slic_unpack_neighbor_keys(const uint64_t* keys_dev, int64_t n, int32_t* idx_
 /* Test hook, host only (no device work): the unit list the symmetric screen would execute for a self-search of n rows
  * as part `part` of `parts` - mode 0: pre-pass + triangle share, 1: row-bests pre-pass only, 2: triangle share only,
  * 3: fused (own rows' pre-pass + triangle share, the multi-GPU kernel); gated_chunks > 0: with upload gates
- * (slic_finch_host); col_tile: column-tile width of the kernel, 128 (A-resident kernels, d_pad <= 512) or 256.
+ * (slic_finch_host).
  * units_out_host [capacity, 6] int32 (optional) receives per unit {row unit, first column tile, tile count, tile stride,
- * gate or -1, column-direction flag}; a unit covers the 256-row x col_tile-column tiles (row unit, first + k * stride),
- * k < count.  Lets a CPU test check that the parts tile the triangle exactly. */
-int slic_debug_sym_plan(int64_t n, int32_t part, int32_t parts, int32_t mode, int32_t gated_chunks, int32_t col_tile,
+ * gate or -1, column-direction flag}; a unit covers the 256 x 256 tiles (row unit, first + k * stride), k < count.
+ * Lets a CPU test check that the parts tile the triangle exactly. */
+int slic_debug_sym_plan(int64_t n, int32_t part, int32_t parts, int32_t mode, int32_t gated_chunks,
                         int32_t* units_out_host, int64_t capacity, int64_t* num_units_out_host);
 
 /* Debug / test hook: raw f16-screen scores of one 128 x 256 tile region, written as float

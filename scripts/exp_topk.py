@@ -1,4 +1,4 @@
-"""Experiment: screen kernel time, top-1 vs top-k, by shape / k / splits (diagnostic)."""
+"""Experiment: screen kernel time, top-1 vs top-k, by shape / k (diagnostic)."""
 import os, sys, ctypes
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -39,9 +39,6 @@ for shape in sys.argv[1:]:
     ms, tf = screen_ms(lambda: be.nn_top1(uq, qb, ux, xb))
     print("%s top1: %.3f ms %.0f TF/s" % (shape, ms, tf), flush=True)
     for k in (1, 20, 50):
-        for sp in os.environ.get("SPLITS", "0").split(","):
-            if sp != "0": os.environ["SLIC_TOPK_SPLITS"] = sp
-            else: os.environ.pop("SLIC_TOPK_SPLITS", None)
-            ms, tf = screen_ms(lambda: be.topk_cosine(uq, ux, k, q_f16=qb, x_f16=xb))
-            st = be.last_stats.cpu().tolist()
-            print("%s top%d splits=%s: %.3f ms %.0f TF/s  reranked/row %.0f listed/row %.0f compactions %d" % (shape, k, sp, ms, tf, st[0] / nq, st[3] * 16.0 / nq, st[2]), flush=True)
+        ms, tf = screen_ms(lambda: be.topk_cosine(uq, ux, k, q_f16=qb, x_f16=xb))
+        st = be.last_stats.cpu().tolist()
+        print("%s top%d: %.3f ms %.0f TF/s  reranked/row %.0f listed/row %.0f compactions %d" % (shape, k, ms, tf, st[0] / nq, st[3] * 16.0 / nq, st[2]), flush=True)

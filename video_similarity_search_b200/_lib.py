@@ -28,7 +28,7 @@ SIGNATURES = {
     "slic_nn_top1": [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i32, _i32, _i32, _i64, _f32, _ptr, _ptr, _ptr, _ptr],
     "slic_sym_row_bests": [_ptr, _ptr, _i64, _i32, _i32, _i32, _i32, _ptr, _ptr],
     "slic_nn_top1_sym_part": [_ptr, _ptr, _i64, _i32, _i32, _i32, _i32, _ptr, _f32, _ptr, _ptr, _ptr],
-    "slic_debug_sym_plan": [_i64, _i32, _i32, _i32, _i32, _i32, _ptr, _i64, _ptr],
+    "slic_debug_sym_plan": [_i64, _i32, _i32, _i32, _i32, _ptr, _i64, _ptr],
     "slic_unpack_neighbor_keys": [_ptr, _i64, _ptr, _ptr, _ptr, _ptr],
     "slic_screen_scores_debug": [_ptr, _i64, _ptr, _i64, _i32, _ptr, _ptr],
     "slic_distance_matrix": [_ptr, _i64, _ptr, _i64, _i32, _i32, _i32, _i32, _ptr, _i64, _ptr],

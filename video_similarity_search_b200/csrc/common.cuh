@@ -89,9 +89,6 @@ struct ScreenPeers {
     int* own_sync;                             // this rank's pre-pass arrival counter (its window)
     unsigned int* peer_best[SLIC_MAX_PEERS];   // the same two of every other rank
     int* peer_sync[SLIC_MAX_PEERS];
-    int* shared_queue;    // optional: ONE unit counter for all ranks (in rank 0's window); every rank then runs the same
-                          // complete unit list and the GPUs balance each other dynamically
-    int* queue_to_zero;   // rank 0: the counter it resets together with its window; other ranks: nullptr
 };
 // can CTAs of the given shape co-reside with the persistent screen kernel of a gated self-search (see nn_screen_tc.cu)
 bool screen_can_overlap_upload(int64_t n, int d_pad, int guest_threads, int guest_regs);

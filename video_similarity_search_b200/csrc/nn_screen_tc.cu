@@ -1,19 +1,29 @@
-// K1-tc: first-neighbour screen on the 5th-generation tensor cores (tcgen05 + TMEM + TMA), with the
-// per-row candidate filter fused into the epilogue so the nq x n score matrix never reaches HBM.
+// K1-tc: first-neighbour / top-k screen on the 5th-generation tensor cores (tcgen05 + TMEM + TMA), with the per-row
+// candidate filter fused into the epilogue so the nq x n score matrix never reaches HBM.
 // Replaces the O(n^2 D) sgemm/dgemm + three n^2 elementwise passes + argmin behind
 // clustering/finch.py:27-29 (sklearn pairwise_distances -> OpenBLAS).
 //
 // Work decomposition
-//   unit  = (128-row query block) x (one of `splits` contiguous column ranges)
-//   tile  = 128 x 256 scores of a unit, K = d_pad in 64-wide slabs (f16, 128-byte swizzled rows)
-//   CTA   = persistent, one per SM, walks units round-robin; 6 warps:
-//           warp 0  TMA producer   : cp.async.bulk.tensor of the A (16 KB) and B (32 KB) slab per stage
-//           warp 1  MMA issuer     : one thread issues tcgen05.mma (M128 N256 K16) x 4 per slab, commits to
-//                                    the stage's "empty" barrier and, per tile, to the accumulator's "full" barrier
-//           warps 2-5 epilogue     : tcgen05.ld 32 columns at a time out of TMEM (two 256-column accumulators,
-//                                    so the filter of tile t overlaps the MMAs of tile t+1)
-//   Concurrent CTAs work on different row blocks of the SAME column range, so every B slab is fetched
-//   from HBM once per wave and served to the other 147 SMs from L2.
+//   tile  = 256 x 256 scores, K = d_pad in 64-wide slabs (f16, 128-byte swizzled rows), computed by a CTA PAIR (cluster
+//           of 2, tcgen05 cta_group::2): each CTA stages its own 128 query rows of A and half of the B slab, and the
+//           leader issues tcgen05.mma M256 N256 K16 that read both halves.  Two 256-column accumulators in TMEM, so the
+//           filter of tile t overlaps the MMAs of tile t + 1.
+//   unit  = a pair's 256 query rows x a run of column tiles (a column split, or an entry of an explicit unit list).
+//   CTA   = persistent, one per SM.  The leader's producer thread draws unit ids from a global counter (dynamic
+//           queue) and hands them to every role of both CTAs through the unit ring (TC_UQ_DEPTH slots in shared
+//           memory, cluster-scope barriers).  10 warps, 11 for the symmetric kernels:
+//           warp 0     TMA producer: A and B slabs into the operand ring (A once per unit when it is resident)
+//           warp 1     MMA issuer (the leader's lane 0): commits to the stage's "empty" and the accumulator's "full" barrier
+//           warps 2-9  epilogue: tcgen05.ld 32 columns at a time out of TMEM; warp w reads TMEM lanes 32 * (w % 4) and
+//                      the 128-column half (w - 2) / 4 of every tile, one thread = one (query row, column half) stream
+//           warp 10    SYM only: publishes the column thresholds of the coming tiles
+//   Concurrent pairs work on different row blocks of the SAME column range, so every B slab is fetched from HBM once per
+//   wave and served to the other SMs from L2.
+//
+// Template axes of nn_screen_kernel (six instantiations):
+//   TOPK  first neighbour, or the k best (per-row score histograms in shared memory)
+//   ARES  d_pad <= 512: the unit's A rows stay resident in shared memory and only B streams; wider rows stream both
+//   SYM   self-search over the upper triangle of tiles, off-diagonal tiles filtered along rows and columns (top-1 only)
 //
 // Fused filter (per query row = one epilogue thread, state in registers)
 //   best = running maximum of the screened scores seen so far; a column is appended to the row's
@@ -25,8 +35,15 @@
 //   kernel - the result never depends on f16 precision.
 //
 // Bound: tensor pipe.  Algorithmic work 2 * nq * n * d_pad flop; HBM traffic ~ (nq + n) * d_pad * 2 bytes.
+//
+// Variants measured and removed (records under profiles/):
+//   128-column tiles with four accumulators: 31.6 against 22.2 ms at C3 (r2_screen_pipeline_trace.txt)
+//   L2 prefetch of the B slabs ahead of the ring: 23.3 -> 24.3 ms at C3 (r2_screen_pipeline_trace.txt)
+//   static unit striding instead of the dynamic queue: round 1 row of r2_screen_pipeline_trace.txt
+//   one box-wide unit queue for a multi-GPU search: slower than fixed shares (r2_runs/exp_sq8.log)
+//   single-CTA 128 x 256 tiles: a third more L2 -> SM operand traffic per flop than a pair (r2_ptxas_table.txt lists them)
+//   column-chunk width of the symmetric plan: 64 tiles is the fastest (r2_runs/exp_chunk.log)
 #include <cuda.h>
-#include <cuda_fp16.h>
 #include <cuda_fp16.h>
 #include <math.h>
 #include <stdlib.h>
@@ -42,50 +59,37 @@
 namespace slic {
 
 constexpr int TC_BM = 128, TC_BK = 64, TC_UMMA_K = 16;
-// Column-tile width.  WIDE (256, what every kernel runs): two 256-column accumulators in TMEM, every epilogue warp filters
-// one 128-column half of EVERY tile - the pair then advances at the pace of the slowest of its 16 epilogue warps on every
-// single tile (measured on the symmetric kernel at C3: MMA busy 66 %, epilogue warps busy 69 %, yet 6 019 cycles per tile
-// against 4 096 of MMA work).  NARROW (128; built, tested, NOT selected - SLIC_SCREEN_NARROW=1 builds a plan for it only in
-// the planner tests): FOUR 128-column accumulators, the epilogue warps in two groups that take ALTERNATE tiles, so that a
-// tile is released by the 8 warps of one group and the MMA issuer runs up to three tiles ahead.  Measured (round 2, C3):
-// the accumulator wait of the MMA issuer drops from 15 % to 5 % as intended, but the kernel takes 31.6 ms instead of 22.2:
-// with both operands in shared memory a tcgen05.mma M256 N128 K16 takes ~113 cycles against ~124 for N256 - the A
-// operand (4 KB per CTA and instruction) is re-read from shared memory by every instruction whatever N is, so halving N
-// halves the flops per instruction at the same cost.  A narrow tile needs A in TMEM, which the four accumulators fill.
-constexpr int TC_BN_WIDE = 256, TC_BN_NARROW = 128;
+// Column-tile width: two 256-column accumulators in TMEM, every epilogue warp filters one 128-column half of EVERY tile.
+constexpr int TC_BN = 256;
 // K slabs per ring stage of the A-resident kernels.  2 = three 32 KB stages, 8 MMAs per barrier round trip.  (1 = six 16 KB
 // stages was measured in round 2 at C3: operand wait of the MMA issuer 15 % -> 25 %, kernel 22.6 -> 24.1 ms: the finer
 // hand-over costs more in round trips than it gains in ring occupancy.)
 constexpr int TC_ARES_SPS = 2;
-constexpr bool TC_NARROW_ARES = false;   // (true: the A-resident kernels run on narrow tiles - the experiment above)
 constexpr int TC_ROW_UNIT = 256;   // rows of a CTA pair's unit (the symmetric planner counts row units and column tiles)
+static_assert(TC_ROW_UNIT == TC_BN, "a row unit's diagonal block is one column tile");
 constexpr uint32_t TC_A_BYTES = TC_BM * TC_BK * 2;   // 16 KB
-// NCTA = 1: one CTA per 128 x 256 tile, it stages the whole 256-column B slab (32 KB).
-// NCTA = 2: a CTA pair (cluster of 2, tcgen05 cta_group::2) works on a 256 x 256 tile; each CTA stages its own 128
-//           query rows of A and HALF of the B slab (16 KB) and the tensor cores of both SMs read both halves, so
-//           the L2 -> SM operand traffic per flop drops by a third and 6 stages fit instead of 4.
-// ARES (pairs only, d_pad <= 512): the unit's A rows (128 x d_pad f16 <= 128 KB) are loaded ONCE per unit and stay
-//           resident; only B slabs stream through the ring.  A is the one operand no other SM shares, so this removes
-//           most of the L2 -> SM traffic that bounds the streaming variants.
+// Each CTA of a pair stages its own 128 query rows of A and HALF of the B slab (16 KB); the tensor cores of both SMs read
+// both halves.
+// ARES (d_pad <= 512): the unit's A rows (128 x d_pad f16 <= 128 KB) are loaded ONCE per unit and stay resident; only B
+//           slabs stream through the ring.  A is the one operand no other SM shares, so this removes most of the
+//           L2 -> SM traffic that bounds the streaming variants.
 constexpr int TC_ARES_MAX_SLABS = 8;
 // barrier block behind the operands: 38 eight-byte slots (pipeline barriers, TMEM slot, log counters, unit ring)
 constexpr uint32_t TC_BAR_BYTES = 384;
 constexpr int TC_UQ_DEPTH = 4;   // unit ring: ids of the units the scheduler has handed out, consumed in order by every role
 constexpr int TC_TMEM_COLS = 512;
-template <int NCTA, bool ARES, bool TOPK> struct TcCfg {
-    static constexpr int BN = (ARES && TC_NARROW_ARES) ? TC_BN_NARROW : TC_BN_WIDE;
-    static constexpr int ACCS = TC_TMEM_COLS / BN;          // accumulators in TMEM: 4 (narrow) or 2 (wide)
-    static constexpr bool GROUPED = BN == TC_BN_NARROW;     // epilogue warps in two groups that take alternate tiles
-    static constexpr uint32_t B_ROWS = BN / NCTA;
+constexpr int TC_ACCS = TC_TMEM_COLS / TC_BN;   // accumulators in TMEM
+template <bool ARES, bool TOPK> struct TcCfg {
+    static constexpr uint32_t B_ROWS = TC_BN / 2;
     static constexpr uint32_t B_BYTES = B_ROWS * TC_BK * 2;
     static constexpr uint32_t A_RES_BYTES = ARES ? TC_ARES_MAX_SLABS * TC_A_BYTES : 0;      // 128 KB
     // K slabs per ring stage: the A-resident top-1 kernel moves two (32 KB of B per CTA and barrier round trip,
     // 8 MMAs per wait / commit); the top-k variant has 32 KB less shared memory and keeps four single-slab stages
-    static constexpr int SPS = NCTA == 2 ? (ARES ? TC_ARES_SPS : 2) : 1;
+    static constexpr int SPS = ARES ? TC_ARES_SPS : 2;
     static constexpr uint32_t SLAB_BYTES = ARES ? B_BYTES : TC_A_BYTES + B_BYTES;   // one K slab of a stage
     static constexpr uint32_t STAGE_BYTES = SPS * SLAB_BYTES;
     // A-resident: 96 KB (64 KB with the top-k histograms) of ring behind the 128 KB of A rows
-    static constexpr int STAGES = ARES ? (TOPK ? 64 : 96) * 1024 / (int)STAGE_BYTES : (NCTA == 1 ? 4 : 3);
+    static constexpr int STAGES = ARES ? (TOPK ? 64 : 96) * 1024 / (int)STAGE_BYTES : 3;
     static_assert(STAGES >= 2 && STAGES <= 6, "ring depth");
     static constexpr uint32_t OPERAND_BYTES = A_RES_BYTES + STAGES * STAGE_BYTES;            // 192 KB, ARES: 192 / 224 KB
     static constexpr uint32_t SMEM_BYTES = OPERAND_BYTES + TC_BAR_BYTES /*barriers, unit ring*/ + 960 /*alignment slack*/ +
@@ -102,7 +106,6 @@ template <int NCTA, bool ARES, bool TOPK> struct TcCfg {
     static_assert(TOPK || SMEM_BYTES <= CORESIDENT_MAX_BYTES,
                   "top-1 variant (gated launches) leaves no shared memory for a co-resident CTA of the upload stream");
     static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB of shared memory a CTA may use");
-    static_assert(!ARES || NCTA == 2, "the A-resident variant exists for CTA pairs only");
 };
 constexpr int TC_MAX_STAGES = 6;
 constexpr int TC_EPI_WARPS = 8;   // two per TMEM lane quadrant: each takes one 128-column half of every tile
@@ -148,10 +151,6 @@ struct ScreenParams {
     // finished when those of split s start, which spares them the listing of their first tile and the whole threshold
     // ramp (~k ln(columns / 128) listings per stream).
     int* cand_tb;
-    // experiment (SLIC_SCREEN_L2PF, default 0 = off): tiles ahead of the ring whose B slabs the producer prefetches into L2.
-    // Measured at C3 with 1 / 2 / 4 tiles: operand wait of the MMA issuer 14.4 % -> 13.8 %, kernel 23.3 -> 24.3 ms - the wait is
-    // L2 -> SM delivery, not DRAM latency (profiles/r2_screen_pipeline_trace.txt).
-    int l2_prefetch;
     float* dump;           // debug: raw scores [nq][n] or nullptr
     int* error_flag;       // set when a barrier wait times out
     unsigned long long* trace;  // optional [8] cycle counters summed over CTAs (diagnostic, see slic_screen_trace)
@@ -175,7 +174,6 @@ struct ScreenParams {
     // Dynamic scheduling: units are handed out in list order from this global counter (zeroed before the launch) to
     // whichever CTA pair becomes free - no pair idles while another still holds a queue of long units.
     int* queue;
-    int queue_on_peer;   // the counter lives in another GPU's window (box-wide queue experiment): system-scope draws
     // Multi-GPU fused search (comm.cu): the pre-pass units of this rank publish their rows' bests into the best arrays
     // of the OTHER ranks as well (red.max over NVLink peer mappings) and count their arrivals on every rank's
     // sync_counter, so the triangle units of every rank start from thresholds for ALL rows - the exchange that used to
@@ -186,7 +184,7 @@ struct ScreenParams {
 };
 
 struct UnitInfo {
-    int64_t row_unit;   // index of the unit's row block (single CTA) or row-block pair
+    int64_t row_unit;   // index of the unit's row-block pair
     int64_t ct0;        // first column tile
     int count, stride;  // tiles ct0 + k * stride, k < count
     int gate;           // -1: none
@@ -366,16 +364,6 @@ __device__ __forceinline__ void counter_wait(const int* counter, int target, int
         }
     }
 }
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint32_t dst, uint32_t bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
-        : "memory");
-}
-// L2 prefetch of one TMA box (no shared-memory destination, no barrier)
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* map, int c0, int c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(map), "r"(c0), "r"(c1) : "memory");
-}
 // shared::cluster address of the same smem offset in the pair's leader CTA (rank 0): clear the peer bit
 constexpr uint32_t TC_PEER_BIT_MASK = 0xFEFFFFFFu;
 __device__ __forceinline__ void tma_load_2d_pair(const CUtensorMap* map, uint32_t dst, uint32_t leader_bar, int c0, int c1) {
@@ -456,18 +444,6 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                          uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                                uint32_t accumulate) {
     asm volatile(
@@ -525,9 +501,7 @@ __device__ __forceinline__ uint64_t umma_smem_desc(uint32_t smem_addr) {
 // kind::f16 instruction descriptor: D=f32 (bits 4-5 = 1), A=B=float16 (format fields at bits 7-9 and 10-12 = 0; 1 would
 // be bfloat16), both K-major, N >> 3 at bits 17-22, M >> 4 at bits 24-28.
 // cta_group::2: the instruction spans both CTAs, M = 256
-__host__ __device__ constexpr uint32_t tc_idesc(int bn, int ncta) {
-    return (1u << 4) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)((ncta * TC_BM) >> 4) << 24);
-}
+constexpr uint32_t TC_IDESC = (1u << 4) | ((uint32_t)(TC_BN >> 3) << 17) | ((uint32_t)((2 * TC_BM) >> 4) << 24);
 
 // ---- candidate list maintenance (slow path, rare) -------------------------------------------
 struct RowState {
@@ -870,13 +844,13 @@ __device__ __forceinline__ void epi_chunk(EpiCtx<TOPK>& cx, uint32_t (&v)[32], i
 // 3 * 32 * 152 = 14 592 leaves 1 792 registers there - one warp of a 128-thread guest CTA (<= 56 registers/thread).
 // (slic_screen_can_overlap_upload checks the built kernels against this arithmetic before a gated launch.)
 constexpr int TC_TOP1_MAX_REGS = 152;
-template <bool TOPK, int NCTA, bool ARES, bool SYM = false>
+template <bool TOPK, bool ARES, bool SYM = false>
 __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(const __grid_constant__ CUtensorMap tmap_q,
                                                                   const __grid_constant__ CUtensorMap tmap_x,
                                                                   const ScreenParams p) {
-    typedef TcCfg<NCTA, ARES, TOPK> Cfg;
+    typedef TcCfg<ARES, TOPK> Cfg;
     constexpr int STAGES = Cfg::STAGES;
-    static_assert(!SYM || (NCTA == 2 && !TOPK), "the symmetric variant exists for the top-1 CTA-pair kernels only");
+    static_assert(!SYM || !TOPK, "the symmetric variant exists for the top-1 kernels only");
     extern __shared__ uint8_t smem_raw[];
     // (the dynamic smem window starts at the same offset in both CTAs of a pair, so the aligned offsets agree)
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -892,20 +866,16 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
         }
     }
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::OPERAND_BYTES);
-    const uint32_t bar_full = smem_u32(bars);                              // [STAGES]  (pair: the leader's are used)
+    const uint32_t bar_full = smem_u32(bars);                              // [STAGES]  (the leader's are used)
     const uint32_t bar_empty = smem_u32(bars + TC_MAX_STAGES);             // [STAGES]
-    constexpr int BN = Cfg::BN, ACCS = Cfg::ACCS;
-    constexpr bool GROUPED = Cfg::GROUPED;
-    // epilogue warps that read (and release) one tile: all eight (each a 128-column half), or the four of one group
-    constexpr int TILE_WARPS = GROUPED ? TC_EPI_WARPS / 2 : TC_EPI_WARPS;
-    const uint32_t bar_acc_full = smem_u32(bars + 12);    // [ACCS <= 4]
-    const uint32_t bar_acc_empty = smem_u32(bars + 16);   // [ACCS <= 4]  (pair: the leader's are used)
+    const uint32_t bar_acc_full = smem_u32(bars + 12);    // [TC_ACCS]
+    const uint32_t bar_acc_empty = smem_u32(bars + 16);   // [TC_ACCS]  (the leader's are used)
     const uint32_t bar_a_full = smem_u32(bars + 20);      // ARES: resident A landed (leader's used)
     const uint32_t bar_a_empty = smem_u32(bars + 21);     // ARES: the unit's MMAs retired
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 22);
     // (slots 24-27: the epilogue warps' log counters, see s_logcnt)
-    const uint32_t bar_thr_full = smem_u32(bars + 28);    // SYM [4]: thresholds of a tile are in place (threshold warp)
-    const uint32_t bar_thr_empty = smem_u32(bars + 32);   // SYM [4]: the tile's epilogue warps of this CTA are done with them
+    const uint32_t bar_thr_full = smem_u32(bars + 28);    // SYM [2]: thresholds of a tile are in place (threshold warp)
+    const uint32_t bar_thr_empty = smem_u32(bars + 32);   // SYM [2]: the tile's epilogue warps of this CTA are done with them
     const uint32_t bar_uq_full = smem_u32(bars + 36);     // [TC_UQ_DEPTH]: ring slot holds a unit id (own CTA's copy)
     const uint32_t bar_uq_empty = smem_u32(bars + 40);    // [TC_UQ_DEPTH]: every role of the pair has read it (leader's used)
     const uint32_t uq_val = smem_u32(bars + 44);          // [TC_UQ_DEPTH] int32 unit ids, -1 = no more units
@@ -915,7 +885,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const bool tracing = p.trace != nullptr;
-    const uint32_t cta_rank = NCTA == 2 ? cluster_ctarank() : 0u;   // 0 = leader: issues the MMAs of the pair
+    const uint32_t cta_rank = cluster_ctarank();   // 0 = leader: issues the MMAs of the pair
 
     if (threadIdx.x == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap_q) : "memory");
@@ -924,45 +894,38 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
             mbar_init(bar_full + 8 * s, 1);    // the (leader's) producer's arrive.expect_tx
             mbar_init(bar_empty + 8 * s, 1);   // one tcgen05.commit
         }
-        for (int a = 0; a < ACCS; ++a) {
+        for (int a = 0; a < TC_ACCS; ++a) {
             mbar_init(bar_acc_full + 8 * a, 1);
-            mbar_init(bar_acc_empty + 8 * a, TILE_WARPS * NCTA);  // one arrive per epilogue warp (of the pair) that reads the tile
+            mbar_init(bar_acc_empty + 8 * a, 2 * TC_EPI_WARPS);  // one arrive per epilogue warp of the pair
         }
         mbar_init(bar_a_full, 1);
         mbar_init(bar_a_empty, 1);
         for (int s = 0; s < TC_UQ_DEPTH; ++s) {
             mbar_init(bar_uq_full + 8 * s, 1);   // the scheduler's arrive
             // readers of a slot, pair-wide: 8 epilogue warps (+ threshold warp) per CTA, the leader's MMA issuer, the peer's producer
-            mbar_init(bar_uq_empty + 8 * s, NCTA * (TC_EPI_WARPS + (SYM ? 1 : 0)) + 1 + (NCTA - 1));
+            mbar_init(bar_uq_empty + 8 * s, 2 * (TC_EPI_WARPS + (SYM ? 1 : 0)) + 2);
         }
         if constexpr (SYM) {
-            for (int b = 0; b < 4; ++b) {
+            for (int b = 0; b < 2; ++b) {
                 mbar_init(bar_thr_full + 8 * b, 1);
-                mbar_init(bar_thr_empty + 8 * b, TILE_WARPS);
+                mbar_init(bar_thr_empty + 8 * b, TC_EPI_WARPS);
             }
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
-        if constexpr (NCTA == 2) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                         "r"(TC_TMEM_COLS)
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                         "r"(TC_TMEM_COLS)
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                     "r"(TC_TMEM_COLS)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
     __syncthreads();
-    if constexpr (NCTA == 2) cluster_sync_all();   // the peer's barriers are initialised before anything remote touches them
+    cluster_sync_all();   // the peer's barriers are initialised before anything remote touches them
     tc_fence_after();
     const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_slot);
 
-    const int64_t n_col_tiles = (p.n + BN - 1) / BN;
+    const int64_t n_col_tiles = (p.n + TC_BN - 1) / TC_BN;
     UnitRing ring;
     ring.full = bar_uq_full;
     ring.val = uq_val;
@@ -977,11 +940,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
             uint32_t phase = 0, a_phase = 0;
             unsigned long long t_wait = 0;
             const bool scheduler = cta_rank == 0;
-            // (p.queue == nullptr: static striding over the CTA pairs - kept for A/B measurements, SLIC_SCREEN_STATIC=1)
-            const int stride_groups = (int)(gridDim.x / NCTA);
-            // (a queue shared by the GPUs of a box lives in one rank's peer-mapped window: the draw is an NVLink atomic)
-            auto draw = [&]() -> int { return p.queue_on_peer ? atomicAdd_system(p.queue, 1) : atomicAdd(p.queue, 1); };
-            int u_next = scheduler ? (p.queue ? draw() : (int)(blockIdx.x / NCTA)) : 0;
+            int u_next = scheduler ? atomicAdd(p.queue, 1) : 0;
             while (true) {
                 int u;
                 if (scheduler) {
@@ -989,7 +948,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                     u = u_next < p.num_units ? u_next : -1;
                     mbar_wait_cluster(bar_uq_empty + 8u * ring.slot, ring.phase ^ 1u, p.error_flag);
 #pragma unroll
-                    for (uint32_t r = 0; r < (uint32_t)NCTA; ++r) {
+                    for (uint32_t r = 0; r < 2u; ++r) {
                         st_cluster_u32(peer_smem_addr(uq_val + 4u * ring.slot, r), (uint32_t)u);
                         mbar_arrive_release_cluster(peer_smem_addr(bar_uq_full + 8u * ring.slot, r));
                     }
@@ -997,13 +956,13 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                         ring.slot = 0;
                         ring.phase ^= 1u;
                     }
-                    if (u >= 0) u_next = p.queue ? draw() : u_next + stride_groups;   // (the round trip overlaps this unit's loads)
+                    if (u >= 0) u_next = atomicAdd(p.queue, 1);   // (the round trip overlaps this unit's loads)
                 } else {
                     u = ring_take(ring, false, p.error_flag);
                 }
                 if (u < 0) break;
                 const UnitInfo ui = unit_info(p, u, n_col_tiles);
-                const int64_t row_block = ui.row_unit * NCTA + cta_rank;
+                const int64_t row_block = ui.row_unit * 2 + cta_rank;
                 if (ui.gate >= 0) gate_wait(p.gates + ui.gate, p.error_flag);
                 if constexpr (SYM) {
                     if (ui.coldir && p.sync_counter)
@@ -1020,35 +979,26 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                 }
                 for (int kt = 0; kt < ui.count; ++kt) {
                     const int64_t ct = ui.ct0 + (int64_t)kt * ui.stride;
-                    if (p.l2_prefetch > 0 && kt + p.l2_prefetch < ui.count) {
-                        const int64_t ctp = ui.ct0 + (int64_t)(kt + p.l2_prefetch) * ui.stride;
-                        for (int ks = 0; ks < p.num_k_slabs; ++ks)
-                            tma_prefetch_l2_2d(&tmap_x, ks * TC_BK, (int)(ctp * BN + cta_rank * Cfg::B_ROWS));
-                    }
                     for (int ks = 0; ks < p.num_k_slabs; ks += Cfg::SPS) {
                         mbar_wait_traced(bar_empty + 8 * stage, phase ^ 1, p.error_flag, t_wait, tracing);
                         const uint32_t a_dst = ring_base + stage * Cfg::STAGE_BYTES;
                         const uint32_t b_dst = ARES ? a_dst : a_dst + TC_A_BYTES;
+                        // both CTAs' bytes complete on the LEADER's full barrier
                         if constexpr (ARES) {
                             const int nsl = min(Cfg::SPS, p.num_k_slabs - ks);
                             if (cta_rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2 * (uint32_t)nsl * Cfg::B_BYTES);
                             for (int j = 0; j < nsl; ++j)
                                 tma_load_2d_pair(&tmap_x, b_dst + j * Cfg::SLAB_BYTES, bar_full + 8 * stage, (ks + j) * TC_BK,
-                                                 (int)(ct * BN + cta_rank * Cfg::B_ROWS));
-                        } else if constexpr (NCTA == 2) {
-                            // both CTAs' bytes complete on the LEADER's full barrier
+                                                 (int)(ct * TC_BN + cta_rank * Cfg::B_ROWS));
+                        } else {
                             const int nsl = min(Cfg::SPS, p.num_k_slabs - ks);
                             if (cta_rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2 * (uint32_t)nsl * Cfg::SLAB_BYTES);
                             for (int j = 0; j < nsl; ++j) {
                                 tma_load_2d_pair(&tmap_q, a_dst + j * Cfg::SLAB_BYTES, bar_full + 8 * stage, (ks + j) * TC_BK,
                                                  (int)(row_block * TC_BM));
                                 tma_load_2d_pair(&tmap_x, b_dst + j * Cfg::SLAB_BYTES, bar_full + 8 * stage, (ks + j) * TC_BK,
-                                                 (int)(ct * BN + cta_rank * Cfg::B_ROWS));
+                                                 (int)(ct * TC_BN + cta_rank * Cfg::B_ROWS));
                             }
-                        } else {
-                            mbar_expect_tx(bar_full + 8 * stage, Cfg::STAGE_BYTES);
-                            tma_load_2d(&tmap_q, a_dst, bar_full + 8 * stage, ks * TC_BK, (int)(row_block * TC_BM));
-                            tma_load_2d(&tmap_x, b_dst, bar_full + 8 * stage, ks * TC_BK, (int)(ct * BN));
                         }
                         if (++stage == STAGES) {
                             stage = 0;
@@ -1084,7 +1034,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                 for (int kt = 0; kt < n_tiles; ++kt) {
                     mbar_wait_traced(bar_acc_empty + 8 * acc, acc_phase ^ 1, p.error_flag, t_acc, tracing);
                     tc_fence_after();
-                    const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
+                    const uint32_t tmem_d = tmem_base + (uint32_t)(acc * TC_BN);
                     for (int ks = 0; ks < p.num_k_slabs; ks += Cfg::SPS) {
                         mbar_wait_traced(bar_full + 8 * stage, phase, p.error_flag, t_smem, tracing);
                         tc_fence_after();
@@ -1098,27 +1048,21 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
 #pragma unroll
                                 for (int k = 0; k < TC_BK / TC_UMMA_K; ++k) {
                                     // advancing 16 f16 = 32 bytes along K inside the swizzle atom: +2 in the address field
-                                    if constexpr (NCTA == 2)
-                                        umma_f16_pair(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), tc_idesc(BN, 2),
-                                                       (uint32_t)((ks | j | k) != 0));
-                                    else
-                                        umma_f16(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), tc_idesc(BN, 1),
+                                    umma_f16_pair(tmem_d, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), TC_IDESC,
                                                   (uint32_t)((ks | j | k) != 0));
                                 }
                             }
                         }
-                        // frees the smem stage (in both CTAs of a pair) once these MMAs retire
-                        if constexpr (NCTA == 2) umma_commit_pair(bar_empty + 8 * stage);
-                        else umma_commit(bar_empty + 8 * stage);
+                        // frees the smem stage (in both CTAs) once these MMAs retire
+                        umma_commit_pair(bar_empty + 8 * stage);
                         if (++stage == STAGES) {
                             stage = 0;
                             phase ^= 1;
                         }
                     }
                     // accumulator complete -> epilogue (of both CTAs)
-                    if constexpr (NCTA == 2) umma_commit_pair(bar_acc_full + 8 * acc);
-                    else umma_commit(bar_acc_full + 8 * acc);
-                    if (++acc == ACCS) {
+                    umma_commit_pair(bar_acc_full + 8 * acc);
+                    if (++acc == TC_ACCS) {
                         acc = 0;
                         acc_phase ^= 1;
                     }
@@ -1138,48 +1082,39 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
         // For every tile strictly right of the diagonal (the epilogue's "column role"): threshold of column c =
         // best score published for row c so far - eps, as float16 rounded DOWN (a lower threshold only adds candidates;
         // 2^-11 against eps = 2^-7), with a finite lower bound (threshold - masked score = +inf, never NaN).
-        // Buffers (1 KB in all): wide tiles - 2 x [256 columns], consumed by all eight epilogue warps of the CTA; narrow
-        // tiles - per epilogue group 2 x [128 columns], consumed by the group's four warps.  `tile_seq` counts EVERY tile the
-        // pair processes (it decides which group takes a narrow tile), cseq[g] the column-role tiles of group g.
+        // Buffers (1 KB in all): 2 x [256 columns], consumed by all eight epilogue warps of the CTA; `cseq` counts the
+        // column-role tiles.
         uint16_t* thr_buf = reinterpret_cast<uint16_t*>(smem + Cfg::OPERAND_BYTES + TC_BAR_BYTES);
         constexpr unsigned ENC_POS_INF = 0xff800000u;
-        constexpr int PER_LANE = BN / 32;
-        constexpr int DIAG_TILES = TC_ROW_UNIT / BN;   // column tiles that make up a row unit's diagonal block
-        unsigned tile_seq = 0, cseq0 = 0u, cseq1 = 0u;   // (two scalars: an indexed array would live in local memory)
+        constexpr int PER_LANE = TC_BN / 32;
+        unsigned cseq = 0u;
         for (int u; (u = ring_take(ring, true, p.error_flag)) >= 0;) {
             const UnitInfo ui = unit_info(p, u, n_col_tiles);
-            if (!ui.coldir) {
-                tile_seq += (unsigned)ui.count;
-                continue;
-            }
+            if (!ui.coldir) continue;
             if (p.sync_counter) {   // published bests of the pre-pass are in place (speed only, as for the epilogue)
                 if (lane == 0) counter_wait(p.sync_counter, __ldg(p.sync_targets + ui.gate + 1), p.error_flag);
                 __syncwarp();
             }
-            for (int kt = 0; kt < ui.count; ++kt, ++tile_seq) {
+            for (int kt = 0; kt < ui.count; ++kt) {
                 const int64_t ct = ui.ct0 + (int64_t)kt * ui.stride;
-                if (ct / DIAG_TILES == ui.row_unit) continue;
-                const int grp = GROUPED ? (int)(tile_seq & 1u) : 0;
-                const unsigned cs = grp ? cseq1 : cseq0;
-                const uint32_t buf = cs & 1u, ph = (cs >> 1) & 1u;
-                const uint32_t bi = (uint32_t)grp * 2u + buf;   // barrier / buffer index
+                if (ct == ui.row_unit) continue;   // the diagonal tile (TC_ROW_UNIT == TC_BN)
+                const uint32_t buf = cseq & 1u, ph = (cseq >> 1) & 1u;
                 unsigned e[PER_LANE];   // fetched first: the L2 round trip overlaps the wait for the buffer
 #pragma unroll
                 for (int j = 0; j < PER_LANE; ++j) {
-                    const int64_t c = ct * BN + lane + 32 * j;
+                    const int64_t c = ct * TC_BN + lane + 32 * j;
                     e[j] = c < p.n ? __ldcg(p.best_enc + c) : ENC_POS_INF;
                 }
-                mbar_wait(bar_thr_empty + 8 * bi, ph ^ 1u, p.error_flag);
-                const uint32_t ta = smem_u32(thr_buf + (GROUPED ? bi * 128u : buf * 256u)) + 2u * lane;
+                mbar_wait(bar_thr_empty + 8 * buf, ph ^ 1u, p.error_flag);
+                const uint32_t ta = smem_u32(thr_buf + buf * 256u) + 2u * lane;
 #pragma unroll
                 for (int j = 0; j < PER_LANE; ++j) {
                     const unsigned short t = __half_as_ushort(__float2half_rd(fmaxf(dec_score(e[j]) - p.eps, -60000.f)));
                     asm volatile("st.shared.b16 [%0], %1;" ::"r"(ta + 64u * j), "h"(t) : "memory");
                 }
                 __syncwarp();
-                if (lane == 0) mbar_arrive(bar_thr_full + 8 * bi);
-                if (grp) ++cseq1;
-                else ++cseq0;
+                if (lane == 0) mbar_arrive(bar_thr_full + 8 * buf);
+                ++cseq;
             }
         }
     } else {
@@ -1187,13 +1122,9 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
         // Warp w reads TMEM lanes [32 * (w % 4), +32) (the hardware's lane window of that warp) and the 128-column
         // half (w - 2) / 4 of every tile: one thread = one (query row, column half) stream with its own list.
         const int quad = warp & 3;
-        // wide tiles: the warp's 128-column half of EVERY tile; narrow tiles: the warp's GROUP - it takes the tiles whose
-        // sequence number (over everything the pair processes, all units) has this parity, all 128 columns of them.
-        // Either way one thread = one (query row, stream) with its own candidate list, 128 columns per tile it takes.
         const int half = (warp - 2) >> 2;
         const int row_in_tile = quad * 32 + lane;
-        unsigned seq_all = 0;   // tiles the pair has been through; accumulator of tile s: s % ACCS, barrier phase (s / ACCS) & 1
-        constexpr unsigned TILE_STEP = GROUPED ? 2u : 1u;   // distance to this warp's next tile
+        unsigned seq_all = 0;   // tiles the pair has been through; accumulator of tile s: s % TC_ACCS, barrier phase (s / TC_ACCS) & 1
         unsigned long long t_full = 0;
         const long long t_begin = tracing ? clock64() : 0;
         EpiCtx<TOPK> cx;
@@ -1204,7 +1135,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
         if constexpr (TOPK) cx.hist = smem + Cfg::OPERAND_BYTES + TC_BAR_BYTES + half * TC_BM + row_in_tile;
         unsigned int* s_logcnt = reinterpret_cast<unsigned int*>(bars + 24) + (warp - 2);   // slots 24-27 of the barrier block
         uint16_t* thr_buf = reinterpret_cast<uint16_t*>(smem + Cfg::OPERAND_BYTES + TC_BAR_BYTES);   // SYM: float16 column thresholds
-        unsigned tile_seq = 0;   // SYM: column-role tiles this warp has taken (wide: of all tiles; narrow: of its group's)
+        unsigned tile_seq = 0;   // SYM: column-role tiles this warp has taken
         const int64_t log_region_id = (int64_t)blockIdx.x * TC_EPI_WARPS + (warp - 2);
         if constexpr (SYM) {
             if (lane == 0) *s_logcnt = 0u;
@@ -1231,7 +1162,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                 }
             }
             if (tracing) t_unit += (unsigned long long)(clock64() - tr0);
-            const int64_t row_block = ui.row_unit * NCTA + cta_rank;
+            const int64_t row_block = ui.row_unit * 2 + cta_rank;
             cx.row = row_block * TC_BM + row_in_tile;
             cx.row_ok = cx.row < p.nq;
             cx.self_col = (p.self_offset >= 0 && cx.row_ok) ? cx.row + p.self_offset : -1;
@@ -1262,24 +1193,22 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
             bool prefetched = false;   // va holds an in-flight load of the coming tile's first chunk
             bool first = true;         // no tile of this unit taken yet
             for (int kt = 0; kt < ui.count; ++kt, ++seq_all) {
-                if (GROUPED && (int)(seq_all & 1u) != half) continue;   // the other group's tile
-                const int acc = (int)(seq_all % (unsigned)ACCS);
-                const uint32_t acc_phase = (seq_all / (unsigned)ACCS) & 1u;
+                const int acc = (int)(seq_all % (unsigned)TC_ACCS);
+                const uint32_t acc_phase = (seq_all / (unsigned)TC_ACCS) & 1u;
                 const int64_t ct = ui.ct0 + (int64_t)kt * ui.stride;
-                const int64_t col0 = GROUPED ? ct * BN : ct * BN + half * 128;
+                const int64_t col0 = ct * TC_BN + half * 128;
                 // SYM: tiles strictly right of the diagonal also serve their columns as queries; their thresholds come from
                 // the threshold warp through shared memory
                 bool cdir = false;
                 uint32_t thr_tile = 0u;   // shared-memory address of this tile's 128 column thresholds
                 uint32_t thr_done_bar = 0u;
                 if constexpr (SYM) {
-                    cdir = ui.coldir && ct / (TC_ROW_UNIT / BN) != ui.row_unit;
+                    cdir = ui.coldir && ct != ui.row_unit;
                     if (cdir) {   // the threshold warp runs two tiles ahead: this wait is normally a single poll
                         const uint32_t buf = tile_seq & 1u, ph = (tile_seq >> 1) & 1u;
-                        const uint32_t bi = GROUPED ? (uint32_t)half * 2u + buf : buf;   // barrier index (see the threshold warp)
-                        thr_tile = smem_u32(thr_buf + (GROUPED ? bi : buf * 2 + half) * 128);
-                        thr_done_bar = bar_thr_empty + 8 * bi;
-                        mbar_wait(bar_thr_full + 8 * bi, ph, p.error_flag);
+                        thr_tile = smem_u32(thr_buf + (buf * 2 + half) * 128);
+                        thr_done_bar = bar_thr_empty + 8 * buf;
+                        mbar_wait(bar_thr_full + 8 * buf, ph, p.error_flag);
                         ++tile_seq;
                     }
                 }
@@ -1289,7 +1218,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                     mbar_wait_traced(bar_acc_full + 8 * acc, acc_phase, p.error_flag, t_full, tracing);
                     tc_fence_after();
                 }
-                const uint32_t tbase = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + (GROUPED ? 0 : half * 128));
+                const uint32_t tbase = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * TC_BN + half * 128);
                 if constexpr (TOPK) {
                     cx.count = !first;
                     if (first) {
@@ -1329,10 +1258,7 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                             // every TMEM read of this accumulator is complete: hand it back before the last filter
                             tc_fence_before();
                             __syncwarp();
-                            if (lane == 0) {
-                                if constexpr (NCTA == 2) mbar_arrive_leader(bar_acc_empty + 8 * acc);
-                                else mbar_arrive(bar_acc_empty + 8 * acc);
-                            }
+                            if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * acc);
                         }
                         epi_chunk<TOPK, false>(cx, va, col0 + 32 * c, plain);
                     }
@@ -1352,22 +1278,19 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
                             // every TMEM read of this accumulator is complete: hand it back before the last filter
                             tc_fence_before();
                             __syncwarp();
-                            if (lane == 0) {
-                                if constexpr (NCTA == 2) mbar_arrive_leader(bar_acc_empty + 8 * acc);
-                                else mbar_arrive(bar_acc_empty + 8 * acc);
-                            }
+                            if (lane == 0) mbar_arrive_leader(bar_acc_empty + 8 * acc);
                             // Cross-tile prefetch: if this warp's NEXT tile of the unit is already complete in its accumulator,
                             // start reading its first chunk now, so that the load's latency (queueing behind the other warps on
                             // the TMEM read port) hides behind the filter of this tile's last chunk instead of being exposed at
                             // every tile boundary.  One poll, warp-uniform decision; a miss falls back to the blocking wait.
-                            if (kt + (int)TILE_STEP < ui.count) {
-                                const unsigned nxt = seq_all + TILE_STEP;
-                                const int acc_n = (int)(nxt % (unsigned)ACCS);
-                                const bool ready = __all_sync(0xffffffffu, mbar_test(bar_acc_full + 8 * acc_n, (nxt / (unsigned)ACCS) & 1u));
+                            if (kt + 1 < ui.count) {
+                                const unsigned nxt = seq_all + 1;
+                                const int acc_n = (int)(nxt % (unsigned)TC_ACCS);
+                                const bool ready = __all_sync(0xffffffffu, mbar_test(bar_acc_full + 8 * acc_n, (nxt / (unsigned)TC_ACCS) & 1u));
                                 if (ready) {
                                     tc_fence_after();
-                                    tmem_ld_issue(tmem_base + ((uint32_t)(quad * 32) << 16) +
-                                                      (uint32_t)(acc_n * BN + (GROUPED ? 0 : half * 128)), va);
+                                    tmem_ld_issue(tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc_n * TC_BN + half * 128),
+                                                  va);
                                     prefetched = true;
                                 }
                             }
@@ -1429,15 +1352,10 @@ __global__ void __maxnreg__(TOPK ? 168 : TC_TOP1_MAX_REGS) nn_screen_kernel(cons
 
     tc_fence_before();
     __syncthreads();
-    if constexpr (NCTA == 2) cluster_sync_all();   // the peer no longer reads this CTA's smem or signals its barriers
+    cluster_sync_all();   // the peer no longer reads this CTA's smem or signals its barriers
     if (warp == 1) {
         tc_fence_after();
-        if constexpr (NCTA == 2)
-            asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS)
-                         : "memory");
-        else
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS)
-                         : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
     }
 }
 
@@ -1700,39 +1618,12 @@ struct ScreenPlan {
     int64_t units;
 };
 
-// CTAs per tile group: 2 (CTA pairs, tcgen05 cta_group::2) unless SLIC_SCREEN_NCTA=1 selects the single-CTA kernel
-static int screen_ncta() {
-    static int cached = 0;
-    if (cached == 0) {
-        const char* e = getenv("SLIC_SCREEN_NCTA");
-        cached = (e && atoi(e) == 1) ? 1 : 2;
-    }
-    return cached;
-}
-
-// SLIC_SCREEN_ARES=0 keeps A streaming (experiments / fallback)
-static bool screen_ares_allowed() {
-    static int cached = -1;
-    if (cached < 0) {
-        const char* e = getenv("SLIC_SCREEN_ARES");
-        cached = (e && atoi(e) == 0) ? 0 : 1;
-    }
-    return cached != 0;
-}
-
-// column-tile width of the kernel a search with this operand width runs on (TcCfg::BN: narrow for the A-resident kernels)
-static int screen_bn(int d_pad) {
-    return (TC_NARROW_ARES && screen_ncta() == 2 && d_pad / TC_BK <= TC_ARES_MAX_SLABS && screen_ares_allowed()) ? TC_BN_NARROW
-                                                                                                                  : TC_BN_WIDE;
-}
-
-static ScreenPlan plan_screen(int64_t nq, int64_t n, int bn) {
-    const int ncta = screen_ncta();
-    const int64_t row_blocks = ceil_div(nq, TC_BM * ncta), col_tiles = ceil_div(n, bn);
-    const int64_t sms = num_sms() / ncta;
-    // enough units for >= ~6 waves when the problem allows it, but keep >= 2048 columns (8 wide tiles) per unit
+static ScreenPlan plan_screen(int64_t nq, int64_t n) {
+    const int64_t row_blocks = ceil_div(nq, TC_ROW_UNIT), col_tiles = ceil_div(n, TC_BN);
+    const int64_t sms = num_sms() / 2;
+    // enough units for >= ~6 waves when the problem allows it, but keep >= 2048 columns (8 tiles) per unit
     int64_t want = ceil_div(6 * sms, row_blocks);
-    const int64_t min_tiles = 8 * (TC_BN_WIDE / bn);
+    const int64_t min_tiles = 8;
     int64_t max_splits = col_tiles / min_tiles > 0 ? col_tiles / min_tiles : 1;
     int64_t splits = want < 1 ? 1 : (want > max_splits ? max_splits : want);
     ScreenPlan pl;
@@ -1745,14 +1636,13 @@ static ScreenPlan plan_screen(int64_t nq, int64_t n, int bn) {
 // Top-k variant: every unit restarts with an empty threshold (its first tile is listed in full and the
 // threshold then tightens like k / columns seen), so units should be as long as the wave structure allows:
 // minimise waves x (tiles per unit + start-up cost in tile times).
-static ScreenPlan plan_screen_topk(int64_t nq, int64_t n, int k, int bn) {
-    const int ncta = screen_ncta();
-    const int64_t row_blocks = ceil_div(nq, TC_BM * ncta), col_tiles = ceil_div(n, bn);
-    const int64_t sms = num_sms() / ncta;
-    const int64_t startup = 6 * (TC_BN_WIDE / bn);   // bootstrap pass + threshold ramp of a unit, in tile times
+static ScreenPlan plan_screen_topk(int64_t nq, int64_t n, int k) {
+    const int64_t row_blocks = ceil_div(nq, TC_ROW_UNIT), col_tiles = ceil_div(n, TC_BN);
+    const int64_t sms = num_sms() / 2;
+    const int64_t startup = 6;   // bootstrap pass + threshold ramp of a unit, in tile times
     int64_t best_s = 1, best_cost = INT64_MAX;
     // a stream (half of a unit's tiles) should see >= ~32 k columns, or its own k-th best says little about the row's
-    const int64_t min_tps = ceil_div((int64_t)32 * k, bn / 2);
+    const int64_t min_tps = ceil_div((int64_t)32 * k, TC_BN / 2);
     // (two passes: the cheapest plan, then the FEWEST splits within 2 % of it - every split is one more pair of candidate
     //  streams per row, each restarting from an empty threshold: measured on 100 000 x 1 000 000 x 1 024, k = 50, 7 splits
     //  of 559 tiles against 3 of 1 303 - equal in this model - run the screen at 0.56 against 0.70 of the tensor peak)
@@ -1774,10 +1664,6 @@ static ScreenPlan plan_screen_topk(int64_t nq, int64_t n, int k, int bn) {
             }
         }
     }
-    if (const char* e = getenv("SLIC_TOPK_SPLITS")) {   // experiments only
-        const int64_t v = atoll(e);
-        if (v >= 1 && v <= col_tiles) best_s = v;
-    }
     ScreenPlan pl;
     pl.tiles_per_split = (int)ceil_div(col_tiles, best_s);
     pl.splits = (int)ceil_div(col_tiles, pl.tiles_per_split);
@@ -1796,19 +1682,18 @@ static int topk_cap(int k, int64_t cols_per_split) {
 }
 
 typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const ScreenParams);
-static void pick_screen_kernel(bool sym, bool ares, int ncta, bool is_topk, KernelFn* fn, size_t* smem_bytes) {
+// A rows resident in shared memory when they fit, streamed with B otherwise
+static bool screen_ares(int d_pad) { return d_pad / TC_BK <= TC_ARES_MAX_SLABS; }
+static void pick_screen_kernel(bool sym, bool ares, bool is_topk, KernelFn* fn, size_t* smem_bytes) {
     if (sym) {
-        *fn = ares ? (KernelFn)nn_screen_kernel<false, 2, true, true> : (KernelFn)nn_screen_kernel<false, 2, false, true>;
-        *smem_bytes = ares ? TcCfg<2, true, false>::SYM_SMEM_BYTES : TcCfg<2, false, false>::SYM_SMEM_BYTES;
+        *fn = ares ? (KernelFn)nn_screen_kernel<false, true, true> : (KernelFn)nn_screen_kernel<false, false, true>;
+        *smem_bytes = ares ? TcCfg<true, false>::SYM_SMEM_BYTES : TcCfg<false, false>::SYM_SMEM_BYTES;
     } else if (ares) {
-        *fn = is_topk ? (KernelFn)nn_screen_kernel<true, 2, true> : (KernelFn)nn_screen_kernel<false, 2, true>;
-        *smem_bytes = is_topk ? TcCfg<2, true, true>::SMEM_BYTES : TcCfg<2, true, false>::SMEM_BYTES;
-    } else if (ncta == 2) {
-        *fn = is_topk ? (KernelFn)nn_screen_kernel<true, 2, false> : (KernelFn)nn_screen_kernel<false, 2, false>;
-        *smem_bytes = is_topk ? TcCfg<2, false, true>::SMEM_BYTES : TcCfg<2, false, false>::SMEM_BYTES;
+        *fn = is_topk ? (KernelFn)nn_screen_kernel<true, true> : (KernelFn)nn_screen_kernel<false, true>;
+        *smem_bytes = is_topk ? TcCfg<true, true>::SMEM_BYTES : TcCfg<true, false>::SMEM_BYTES;
     } else {
-        *fn = is_topk ? (KernelFn)nn_screen_kernel<true, 1, false> : (KernelFn)nn_screen_kernel<false, 1, false>;
-        *smem_bytes = is_topk ? TcCfg<1, false, true>::SMEM_BYTES : TcCfg<1, false, false>::SMEM_BYTES;
+        *fn = is_topk ? (KernelFn)nn_screen_kernel<true, false> : (KernelFn)nn_screen_kernel<false, false>;
+        *smem_bytes = is_topk ? TcCfg<false, true>::SMEM_BYTES : TcCfg<false, false>::SMEM_BYTES;
     }
 }
 
@@ -1839,13 +1724,11 @@ static int launch_screen(const uint16_t* q_f16, int64_t nq, const uint16_t* x_f1
                          float* cand_kth = nullptr, const int4* unit_table = nullptr, const int* gates = nullptr,
                          unsigned int* best_enc = nullptr, int64_t exec_tiles = 0, int* log_q = nullptr,
                          int log_region = 0, int* sync_counter = nullptr, const int* sync_targets = nullptr,
-                         const ScreenPeers* peers = nullptr, int* cand_tb = nullptr, int* shared_queue = nullptr) {
-    const int ncta = screen_ncta();
+                         const ScreenPeers* peers = nullptr, int* cand_tb = nullptr) {
     if (gates) SLIC_PROPAGATE(arm_timeout_record());
     CUtensorMap tq, tx;
     SLIC_PROPAGATE(make_tmap(&tq, q_f16, nq, d_pad, TC_BM));
-    const int bn = screen_bn(d_pad);
-    SLIC_PROPAGATE(make_tmap(&tx, x_f16, n, d_pad, bn / ncta));
+    SLIC_PROPAGATE(make_tmap(&tx, x_f16, n, d_pad, TC_BN / 2));
     ScreenParams p;
     p.nq = nq;
     p.n = n;
@@ -1863,15 +1746,6 @@ static int launch_screen(const uint16_t* q_f16, int64_t nq, const uint16_t* x_f1
     p.topk = topk;
     p.cand_kth = cand_kth;
     p.cand_tb = cand_tb;
-    {
-        static int l2pf = -1;   // experiments: SLIC_SCREEN_L2PF=<tiles ahead> (default 0 = off)
-        if (l2pf < 0) {
-            const char* e = getenv("SLIC_SCREEN_L2PF");
-            l2pf = e ? atoi(e) : 0;
-            if (l2pf < 0 || l2pf > 16) l2pf = 0;
-        }
-        p.l2_prefetch = l2pf;
-    }
     p.dump = dump;
     p.error_flag = error_flag;
     p.trace = g_trace;
@@ -1895,42 +1769,29 @@ static int launch_screen(const uint16_t* q_f16, int64_t nq, const uint16_t* x_f1
         }
     }
     Scratch queue;   // (freed in stream order, i.e. after the kernel)
-    p.queue_on_peer = shared_queue ? 1 : 0;
-    if (shared_queue) {
-        p.queue = shared_queue;   // one queue for all GPUs of the box (zeroed by its owner before the cross-rank barrier)
-    } else {
-        SLIC_CUDA_OK(queue.alloc(sizeof(int), st));
-        SLIC_CUDA_OK(cudaMemsetAsync(queue.ptr, 0, sizeof(int), st));
-        p.queue = queue.as<int>();
-    }
-    {
-        static int static_sched = -1;
-        if (static_sched < 0) {
-            const char* e = getenv("SLIC_SCREEN_STATIC");
-            static_sched = e && atoi(e) == 1 ? 1 : 0;
-        }
-        if (static_sched && !shared_queue) p.queue = nullptr;
-    }
+    SLIC_CUDA_OK(queue.alloc(sizeof(int), st));
+    SLIC_CUDA_OK(cudaMemsetAsync(queue.ptr, 0, sizeof(int), st));
+    p.queue = queue.as<int>();
     const bool sym = best_enc != nullptr;
     const bool is_topk = topk > 0;
-    const bool ares = ncta == 2 && p.num_k_slabs <= TC_ARES_MAX_SLABS && screen_ares_allowed();
-    if (sym && (ncta != 2 || is_topk || !unit_table)) {
-        set_error("symmetric screen: needs the CTA-pair top-1 kernel and a unit list");
+    const bool ares = screen_ares(d_pad);
+    if (sym && (is_topk || !unit_table)) {
+        set_error("symmetric screen: needs the top-1 kernel and a unit list");
         return SLIC_ERR_UNSUPPORTED;
     }
     KernelFn fn;
     size_t smem_bytes;
-    pick_screen_kernel(sym, ares, ncta, is_topk, &fn, &smem_bytes);
-    static bool attr_done[64][16] = {{false}};
+    pick_screen_kernel(sym, ares, is_topk, &fn, &smem_bytes);
+    static bool attr_done[64][8] = {{false}};
     int dev = 0;
     SLIC_CUDA_OK(cudaGetDevice(&dev));
-    bool& attr_set = attr_done[dev & 63][(sym ? 8 : 0) + (ares ? 4 : 0) + (ncta == 2 ? 2 : 0) + (is_topk ? 1 : 0)];
+    bool& attr_set = attr_done[dev & 63][(sym ? 4 : 0) + (ares ? 2 : 0) + (is_topk ? 1 : 0)];
     if (!attr_set) {
         SLIC_CUDA_OK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
         attr_set = true;
     }
-    const int64_t groups = num_sms() / ncta;
-    const int64_t grid = (pl.units < groups ? pl.units : groups) * ncta;
+    const int64_t pairs = num_sms() / 2;
+    const int64_t grid = (pl.units < pairs ? pl.units : pairs) * 2;
     if (g_profile) {
         if (!g_ev_start) {
             SLIC_CUDA_OK(cudaEventCreate(&g_ev_start));
@@ -1945,7 +1806,7 @@ static int launch_screen(const uint16_t* q_f16, int64_t nq, const uint16_t* x_f1
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)ncta;
+    attr[0].val.clusterDim.x = 2;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
@@ -1955,7 +1816,7 @@ static int launch_screen(const uint16_t* q_f16, int64_t nq, const uint16_t* x_f1
     if (g_profile) {
         SLIC_CUDA_OK(cudaEventRecord(g_ev_stop, st));
         g_last_flop = 2.0 * (double)nq * (double)n * (double)d_pad;
-        g_last_exec_flop = exec_tiles > 0 ? 2.0 * (double)exec_tiles * (TC_BM * ncta) * bn * (double)d_pad : g_last_flop;
+        g_last_exec_flop = exec_tiles > 0 ? 2.0 * (double)exec_tiles * TC_ROW_UNIT * TC_BN * (double)d_pad : g_last_flop;
         g_have_sample = true;
     }
     return SLIC_OK;
@@ -2031,14 +1892,12 @@ constexpr int SYM_SAMPLE_TILES = 16;
 //                     arrivals of ALL ranks (*prepass_units_all = their number over all parts)
 enum SymMode { SYM_FULL = 0, SYM_BESTS = 1, SYM_TRIANGLE = 2, SYM_FUSED = 3 };
 constexpr int SYM_FUSED_PRE_TILES = 16;   // fused pre-pass: a row unit's sample is cut into units of this many tiles (balance)
-static int plan_screen_sym(int64_t n, int bn, int part, int parts, const GateSpec* g, ScreenPlan* pl,
-                           std::vector<int4>* table, SymMode mode = SYM_FULL, int64_t* prepass_units_all = nullptr,
-                           bool whole_list = false /* SYM_FUSED: the units of ALL parts (shared queue) */) {
+static int plan_screen_sym(int64_t n, int part, int parts, const GateSpec* g, ScreenPlan* pl, std::vector<int4>* table,
+                           SymMode mode = SYM_FULL, int64_t* prepass_units_all = nullptr) {
     const bool own_rows_prepass = mode == SYM_BESTS || mode == SYM_FUSED;
-    // R row units of 256 rows (a CTA pair's rows), T column tiles of bn columns, tpr = column tiles per row unit: the
-    // diagonal block of row unit r is made of column tiles [r * tpr, (r + 1) * tpr) and is filtered along rows only
-    const int tpr = TC_ROW_UNIT / bn;
-    const int64_t R = ceil_div(n, TC_ROW_UNIT), T = ceil_div(n, bn);
+    // R row units of 256 rows (a CTA pair's rows), T column tiles of 256 columns: the diagonal block of row unit r is
+    // column tile r and is filtered along rows only
+    const int64_t R = ceil_div(n, TC_ROW_UNIT), T = ceil_div(n, TC_BN);
     SLIC_REQUIRE(T < 65536, "symmetric screen: too many column tiles");
     SLIC_REQUIRE(parts >= 1 && part >= 0 && part < parts, "symmetric screen: bad partition");
     int64_t chunk_tiles_gate = 0, chunk_units_gate = 0;
@@ -2047,44 +1906,28 @@ static int plan_screen_sym(int64_t n, int bn, int part, int parts, const GateSpe
                          g->chunk_rows % TC_ROW_UNIT == 0,
                      "gated screen: chunk_rows must be a positive multiple of 256");
         SLIC_REQUIRE(ceil_div(n, g->chunk_rows) == g->num_chunks, "gated screen: chunks do not tile the database");
-        chunk_tiles_gate = g->chunk_rows / bn;
+        chunk_tiles_gate = g->chunk_rows / TC_BN;
         chunk_units_gate = g->chunk_rows / TC_ROW_UNIT;
     }
-    static int nocol = -1;   // experiments: SLIC_SYM_NOCOL=1 (wrong results, timing only)
-    if (nocol < 0) {
-        const char* f = getenv("SLIC_SYM_NOCOL");
-        nocol = f && atoi(f) == 1 ? 1 : 0;
-    }
     table->clear();
-    // pre-pass sample: tiles spread over the whole matrix, or over the first upload chunk when the rest is in flight.
-    // Sample sizes are stated in 256-column blocks (the numbers below were measured with wide tiles) and converted.
+    // pre-pass sample: tiles spread over the whole matrix, or over the first upload chunk when the rest is in flight
     const int64_t span = g ? (chunk_tiles_gate < T ? chunk_tiles_gate : T) : T;
-    const int64_t span_w = span / tpr > 0 ? span / tpr : 1;
     // SYM_BESTS / SYM_FUSED: every part pays a warm-up of loose thresholds at the start of its (short) share of the
     // triangle, so a stronger sample pays off from 4 parts on.  Round 1 (bfloat16 screen, eps 2^-7), 8 parts, C3: 16 / 32 /
     // 64 blocks -> 3.96 / 3.64 / 3.30 ms for the triangle share against +0.1 ms per 16 blocks here: 64.  Round 2 (float16,
     // eps 2^-9 + 2^-10: a loose threshold admits far fewer candidates), 4 parts, whole level-0 stage: 7.35 / 7.17 / 7.37 ms:
     // flat, 32.
-    int samples_w = own_rows_prepass ? (parts >= 4 ? 2 * SYM_SAMPLE_TILES : SYM_SAMPLE_TILES) : SYM_SAMPLE_TILES / parts;
-    if (own_rows_prepass && samples_w > span_w / 4) samples_w = (int)(span_w / 4);   // small inputs: a sample, not the whole square
+    int samples = own_rows_prepass ? (parts >= 4 ? 2 * SYM_SAMPLE_TILES : SYM_SAMPLE_TILES) : SYM_SAMPLE_TILES / parts;
+    if (own_rows_prepass && samples > span / 4) samples = (int)(span / 4);   // small inputs: a sample, not the whole square
     // small inputs (a hierarchy's level 1): the pre-pass must stay a sample - measured at 21 436 x 512 float64 centroids:
     // 16 / 10 / 4 sample blocks -> 0.88 / 0.79 / 0.72 ms for the whole search
-    if (mode == SYM_FULL && R < 128 && samples_w > R / 16) samples_w = (int)(R / 16);
-    if (samples_w < 4) samples_w = 4;
-    if (const char* e = getenv("SLIC_SYM_SAMPLES")) {   // experiments only
-        const int v = atoi(e);
-        if (v >= 1 && v <= 64) samples_w = v;
-    }
-    int samples = samples_w * tpr;
+    if (mode == SYM_FULL && R < 128 && samples > R / 16) samples = (int)(R / 16);
+    if (samples < 4) samples = 4;
     if (samples > span) samples = (int)span;
     const int stride = (int)(span / samples);
-    const int64_t pre0 = (own_rows_prepass && !whole_list) ? R * part / parts : 0;
-    const int64_t pre1 = (own_rows_prepass && !whole_list) ? R * (part + 1) / parts : R;
-    int pre_len = mode == SYM_FUSED ? SYM_FUSED_PRE_TILES * tpr : samples;
-    if (const char* e = getenv("SLIC_SYM_PRE_TILES")) {   // experiments only (fused pre-pass unit, in 256-column blocks)
-        const int v = atoi(e);
-        if (mode == SYM_FUSED && v >= 1 && v <= 64) pre_len = v * tpr;
-    }
+    const int64_t pre0 = own_rows_prepass ? R * part / parts : 0;
+    const int64_t pre1 = own_rows_prepass ? R * (part + 1) / parts : R;
+    const int pre_len = mode == SYM_FUSED ? SYM_FUSED_PRE_TILES : samples;
     if (prepass_units_all) *prepass_units_all = R * ceil_div(samples, pre_len);
     for (int64_t r = pre0; r < pre1 && mode != SYM_TRIANGLE; ++r) {
         const int gate = g ? (int)(r / chunk_units_gate) : -1;
@@ -2095,37 +1938,29 @@ static int plan_screen_sym(int64_t n, int bn, int part, int parts, const GateSpe
     // part / parts: a CONTIGUOUS range of the chunk-major unit list holding 1 / parts of the triangle's tiles.  (Dealing
     // the units round-robin was measured at 8 ranks: a rank's 74 concurrent CTA pairs then span ~9 column chunks, the B
     // tiles are no longer shared through L2 and the kernel runs at half speed.)
-    int64_t chunk_tiles = (int64_t)SYM_CHUNK_TILES * tpr;   // 16 384 columns = 16 MB of f16 B rows at d_pad 512
-    if (const char* e = getenv("SLIC_SYM_CHUNK_TILES")) {   // experiments only (in 256-column blocks)
-        const int v = atoi(e);
-        if (v >= 8 && v <= 1024) chunk_tiles = (int64_t)v * tpr;
-    }
+    const int64_t chunk_tiles = SYM_CHUNK_TILES;   // 16 384 columns = 16 MB of f16 B rows at d_pad 512
     int64_t total_tiles = 0;
     for (int64_t c0 = 0; c0 < T; c0 += chunk_tiles) {
         const int64_t c1 = c0 + chunk_tiles < T ? c0 + chunk_tiles : T;
-        for (int64_t r = 0; r * tpr < c1; ++r) total_tiles += c1 - (r * tpr > c0 ? r * tpr : c0);
+        for (int64_t r = 0; r < c1; ++r) total_tiles += c1 - (r > c0 ? r : c0);
     }
     // Unit length: units are handed out dynamically (p.queue), so the last ones to finish leave at most one unit of
     // idle time per CTA pair - keep a unit well below a pair's share of the work (level 1 of a hierarchy has ~60 blocks per
     // pair in total), but long enough to amortise the reload of the resident A rows (one block's worth of traffic).
     const int64_t pairs = num_sms() / 2 > 0 ? num_sms() / 2 : 1;
     int64_t unit_len = total_tiles / parts / (pairs * 12);
-    unit_len = unit_len < 8 * tpr ? 8 * tpr : (unit_len > chunk_tiles ? chunk_tiles : unit_len);
-    if (const char* e = getenv("SLIC_SYM_UNIT_TILES")) {   // experiments only (in 256-column blocks)
-        const int v = atoi(e);
-        if (v >= 1 && v <= SYM_CHUNK_TILES && (int64_t)v * tpr <= chunk_tiles) unit_len = (int64_t)v * tpr;
-    }
+    unit_len = unit_len < 8 ? 8 : (unit_len > chunk_tiles ? chunk_tiles : unit_len);
     int64_t seen_tiles = 0;
     for (int64_t c0 = 0; c0 < T && mode != SYM_BESTS; c0 += chunk_tiles) {
         const int64_t c1 = c0 + chunk_tiles < T ? c0 + chunk_tiles : T;
-        for (int64_t r = 0; r * tpr < c1; ++r) {
+        for (int64_t r = 0; r < c1; ++r) {
             const int gate = g ? (int)((c1 - 1) / chunk_tiles_gate) : -1;   // column chunk >= row chunk
-            for (int64_t ct0 = r * tpr > c0 ? r * tpr : c0; ct0 < c1; ct0 += unit_len) {
+            for (int64_t ct0 = r > c0 ? r : c0; ct0 < c1; ct0 += unit_len) {
                 const int64_t cnt = c1 - ct0 < unit_len ? c1 - ct0 : unit_len;
                 const int64_t owner = seen_tiles * parts / total_tiles;   // < parts: seen_tiles < total_tiles here
                 seen_tiles += cnt;
-                if (owner != part && !whole_list) continue;
-                table->push_back(unit_entry(r, ct0, (int)cnt, 1, gate, 0, nocol == 0));
+                if (owner != part) continue;
+                table->push_back(unit_entry(r, ct0, (int)cnt, 1, gate, 0, true));
             }
         }
     }
@@ -2137,16 +1972,15 @@ static int plan_screen_sym(int64_t n, int bn, int part, int parts, const GateSpe
     return SLIC_OK;
 }
 
-static int plan_screen_gated(int64_t nq, int64_t n, int bn, int64_t self_offset, const GateSpec& g, ScreenPlan* pl,
+static int plan_screen_gated(int64_t nq, int64_t n, int64_t self_offset, const GateSpec& g, ScreenPlan* pl,
                              std::vector<int4>* table) {
-    const int ncta = screen_ncta();
-    const int64_t rows_per_unit = (int64_t)TC_BM * ncta;
+    const int64_t rows_per_unit = TC_ROW_UNIT;
     SLIC_REQUIRE(g.gates && g.num_chunks >= 1 && g.num_chunks < 32768 && g.chunk_rows > 0 && g.chunk_rows % TC_ROW_UNIT == 0,
                  "gated screen: chunk_rows must be a positive multiple of 256");
     SLIC_REQUIRE(ceil_div(n, g.chunk_rows) == g.num_chunks, "gated screen: chunks do not tile the database");
     SLIC_REQUIRE(self_offset >= 0 && self_offset + nq <= n, "gated screen: queries must be database rows");
     const int64_t row_units = ceil_div(nq, rows_per_unit);
-    pl->tiles_per_split = (int)(g.chunk_rows / bn);
+    pl->tiles_per_split = (int)(g.chunk_rows / TC_BN);
     pl->splits = g.num_chunks;
     pl->units = row_units * pl->splits;
     table->clear();
@@ -2160,7 +1994,7 @@ static int plan_screen_gated(int64_t nq, int64_t n, int bn, int64_t self_offset,
                 const int need = rc > s ? rc : s;
                 if (need != gate) continue;
                 const int64_t ct0 = (int64_t)s * pl->tiles_per_split;
-                int64_t cnt = ceil_div(n, bn) - ct0;
+                int64_t cnt = ceil_div(n, TC_BN) - ct0;
                 if (cnt > pl->tiles_per_split) cnt = pl->tiles_per_split;
                 table->push_back(unit_entry(r, ct0, (int)cnt, 1, gate, s, false));
             }
@@ -2194,11 +2028,11 @@ static int nn_top1_impl(const T* q_unit, const uint16_t* q_f16, int64_t nq, cons
         gate = nullptr;
         after = nullptr;
     }
-    ScreenPlan pl = plan_screen(nq, n, screen_bn(d_pad));
+    ScreenPlan pl = plan_screen(nq, n);
     std::vector<int4> table;
     Scratch table_dev;
     if (gate) {
-        SLIC_PROPAGATE(plan_screen_gated(nq, n, screen_bn(d_pad), self_offset, *gate, &pl, &table));
+        SLIC_PROPAGATE(plan_screen_gated(nq, n, self_offset, *gate, &pl, &table));
         SLIC_CUDA_OK(table_dev.alloc(table.size() * sizeof(int4), st));
         SLIC_PROPAGATE(stage_to_device(table_dev.ptr, table.data(), table.size() * sizeof(int4), st));
     }
@@ -2252,8 +2086,8 @@ template <typename T>
 static int topk_tc_impl(const T* q_unit, const uint16_t* q_f16, int64_t nq, const T* x_unit, const uint16_t* x_f16,
                         int64_t n, int d, int d_pad, int k, int64_t self_offset, float eps, int* idx_out, T* dist_out,
                         int* stats_out, cudaStream_t st) {
-    const ScreenPlan pl = plan_screen_topk(nq, n, k, screen_bn(d_pad));
-    const int TC_CAP_TOPK = topk_cap(k, (int64_t)pl.tiles_per_split * (screen_bn(d_pad) / 2));
+    const ScreenPlan pl = plan_screen_topk(nq, n, k);
+    const int TC_CAP_TOPK = topk_cap(k, (int64_t)pl.tiles_per_split * (TC_BN / 2));
     const int64_t slots = (int64_t)pl.splits * 2 * nq;   // one list per (split, 128-column half of the tiles, row)
     Scratch ci, cs, cc, cf, ck, ctb, ovr, stats;
     SLIC_CUDA_OK(ctb.alloc(slots * sizeof(int), st));
@@ -2311,7 +2145,7 @@ static bool screen_sym_allowed() {
         const char* e = getenv("SLIC_SCREEN_SYM");
         cached = (e && atoi(e) == 0) ? 0 : 1;
     }
-    return cached != 0 && screen_ncta() == 2;
+    return cached != 0;
 }
 
 // order-preserving score encoding <-> the same order as SIGNED int32 (what an all-reduce MAX over int32 compares)
@@ -2324,11 +2158,10 @@ __global__ void flip_sign_bit_kernel(const unsigned int* __restrict__ in, int64_
 __global__ void sym_init_kernel(int* __restrict__ stats8, int* __restrict__ lcnt, int64_t regions,
                                 unsigned char* __restrict__ rmin_bytes, int64_t rmin_n_bytes, int* __restrict__ sync_counter,
                                 unsigned int* __restrict__ best, const unsigned int* __restrict__ bests_in, int64_t n,
-                                unsigned int* __restrict__ idx_out, int* __restrict__ queue_to_zero) {
+                                unsigned int* __restrict__ idx_out) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < 8) stats8[i] = 0;
     if (i == 0) *sync_counter = 0;
-    if (i == 0 && queue_to_zero) *queue_to_zero = 0;
     if (i < regions) lcnt[i] = 0;
     if (i < n) {
         best[i] = bests_in ? (bests_in[i] ^ 0x80000000u) : ENC_NEG_INF;   // exchanged bests arrive in signed-comparable form
@@ -2448,11 +2281,7 @@ static int nn_top1_sym_impl(const T* unit, const uint16_t* ub, int64_t n, int d,
     ScreenPlan pl;
     std::vector<int4> table;
     int64_t prepass_units_all = 0;
-    // fused multi-GPU search with ONE unit queue for the box: every rank holds the same complete list (all rows' pre-pass,
-    // the whole triangle) and draws from the shared counter - the GPUs balance each other as the CTA pairs of one GPU do
-    const bool shared_list = peers && peers->shared_queue;
-    SLIC_PROPAGATE(plan_screen_sym(n, screen_bn(d_pad), part, parts, gate, &pl, &table, (SymMode)mode, &prepass_units_all,
-                                   shared_list));
+    SLIC_PROPAGATE(plan_screen_sym(n, part, parts, gate, &pl, &table, (SymMode)mode, &prepass_units_all));
     SLIC_REQUIRE((mode == SYM_FUSED) == (peers != nullptr), "symmetric screen: the fused mode needs peer windows (and only it)");
     SLIC_REQUIRE(mode != SYM_FUSED || (stats_ext && !gate), "symmetric screen: the fused mode is asynchronous and ungated");
     int64_t exec_tiles = 0;
@@ -2511,21 +2340,14 @@ static int nn_top1_sym_impl(const T* unit, const uint16_t* ub, int64_t n, int d,
         sym_init_kernel<<<(unsigned)ceil_div(threads, 256), 256, 0, st>>>(stats_dev, lcnt.as<int>(), regions,
                                                                          static_cast<unsigned char*>(rmin.ptr), rmin_bytes,
                                                                          sync_counter_dev, best_dev,
-                                                                         (const unsigned int*)bests_in, n, (unsigned int*)idx_out,
-                                                                         peers ? peers->queue_to_zero : nullptr);
+                                                                         (const unsigned int*)bests_in, n, (unsigned int*)idx_out);
         SLIC_LAUNCH_OK();
     }
     if (before_screen) SLIC_PROPAGATE(before_screen(before_ctx));
-    static int nowait = -1;   // experiments: SLIC_SYM_NOWAIT=1 lets triangle units start before the pre-pass has finished
-    if (nowait < 0) {
-        const char* e = getenv("SLIC_SYM_NOWAIT");
-        nowait = e && atoi(e) == 1 ? 1 : 0;
-    }
     SLIC_PROPAGATE(launch_screen(ub, n, ub, n, d_pad, 0, eps, 0, pl, lnb.as<int>(), ls.as<float>(), lcnt.as<int>(),
                                  flag_dev, nullptr, stats_dev + 4, st, 0, nullptr, table_dev.as<int4>(),
                                  gate ? gate->gates : nullptr, best_dev, exec_tiles, lq.as<int>(),
-                                 (int)region, nowait ? nullptr : sync_counter_dev, sync_dev + 1, peers, nullptr,
-                                 shared_list ? peers->shared_queue : nullptr));
+                                 (int)region, sync_counter_dev, sync_dev + 1, peers));
     if (g_profile && parts > 1) g_last_flop /= (double)parts;   // this process's share of the algorithmic 2 n^2 d
     if (after) SLIC_PROPAGATE(after(after_ctx));
     if (mode == SYM_BESTS) {   // phase 1 of the multi-GPU search: the row bests are the result, the log is discarded
@@ -2634,12 +2456,10 @@ __global__ void sym_unpack_keys_kernel(const unsigned long long* __restrict__ ke
 // 228 KB of shared memory with 1 KB reserved per resident CTA; 4 sub-partitions of 16 384 registers, warps dealt
 // round-robin, registers allocated per warp in units of 8 per thread.  false -> the caller uploads first, then searches.
 bool screen_can_overlap_upload(int64_t n, int d_pad, int guest_threads, int guest_regs) {
-    const int ncta = screen_ncta();
     const bool sym = screen_self_search_is_symmetric(n);
-    const bool ares = ncta == 2 && d_pad / TC_BK <= TC_ARES_MAX_SLABS && screen_ares_allowed();
     KernelFn fn;
     size_t smem_bytes;
-    pick_screen_kernel(sym, ares, ncta, false, &fn, &smem_bytes);
+    pick_screen_kernel(sym, screen_ares(d_pad), false, &fn, &smem_bytes);
     cudaFuncAttributes fa;
     if (cudaFuncGetAttributes(&fa, fn) != cudaSuccess) {
         cudaGetLastError();
@@ -2767,11 +2587,10 @@ int slic_nn_top1_sym_part(const float* unit_dev, const uint16_t* f16_dev, int64_
     return SLIC_OK;
 }
 
-int slic_debug_sym_plan(int64_t n, int32_t part, int32_t parts, int32_t mode, int32_t gated_chunks, int32_t col_tile,
-                        int32_t* units_out_host, int64_t capacity, int64_t* num_units_out_host) {
+int slic_debug_sym_plan(int64_t n, int32_t part, int32_t parts, int32_t mode, int32_t gated_chunks, int32_t* units_out_host,
+                        int64_t capacity, int64_t* num_units_out_host) {
     using namespace slic;
     SLIC_REQUIRE(n > 1 && n < ((int64_t)1 << 31) && num_units_out_host, "debug_sym_plan: bad arguments");
-    SLIC_REQUIRE(col_tile == TC_BN_NARROW || col_tile == TC_BN_WIDE, "debug_sym_plan: col_tile must be 128 or 256");
     SLIC_REQUIRE(mode >= 0 && mode <= 3, "debug_sym_plan: mode must be 0 (full), 1 (row bests), 2 (triangle) or 3 (fused)");
     SLIC_REQUIRE(gated_chunks >= 0 && gated_chunks < 4095, "debug_sym_plan: bad chunk count");
     GateSpec gs = {reinterpret_cast<const int*>(num_units_out_host) /* never dereferenced by the planner */, 0, 0};
@@ -2781,7 +2600,7 @@ int slic_debug_sym_plan(int64_t n, int32_t part, int32_t parts, int32_t mode, in
     }
     ScreenPlan pl;
     std::vector<int4> table;
-    SLIC_PROPAGATE(plan_screen_sym(n, col_tile, part, parts, gated_chunks > 0 ? &gs : nullptr, &pl, &table, (SymMode)mode));
+    SLIC_PROPAGATE(plan_screen_sym(n, part, parts, gated_chunks > 0 ? &gs : nullptr, &pl, &table, (SymMode)mode));
     *num_units_out_host = (int64_t)table.size();
     if (units_out_host) {
         SLIC_REQUIRE(capacity >= (int64_t)table.size(), "debug_sym_plan: unit buffer too small");
@@ -2885,8 +2704,8 @@ int slic_screen_scores_debug(const uint16_t* q_f16_dev, int64_t nq, const uint16
     SLIC_REQUIRE(q_f16_dev && x_f16_dev && out_dev, "screen_scores_debug: null pointer");
     SLIC_PROPAGATE(slic_require_device());
     cudaStream_t st = as_stream(stream);
-    const ScreenPlan pl = plan_screen(nq, n, screen_bn(d_pad));
-    const int64_t slots = (int64_t)pl.splits * 2 * nq;   // one list per (split, stream of the row: column half / tile group)
+    const ScreenPlan pl = plan_screen(nq, n);
+    const int64_t slots = (int64_t)pl.splits * 2 * nq;   // one list per (split, 128-column half of the tiles, row)
     Scratch ci, cs, cc, cf, err;
     SLIC_CUDA_OK(ci.alloc(slots * TC_CAP * sizeof(int), st));
     SLIC_CUDA_OK(cs.alloc(slots * TC_CAP * sizeof(float), st));
