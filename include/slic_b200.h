@@ -106,7 +106,8 @@ int slic_nn_exact_top1(const void* q_unit_dev, const int32_t* q_rows_dev, int64_
  * fused per-row candidate filter (scores never leave the SM) followed by an exact re-rank of
  * the surviving candidates in `dtype`.  eps is the screen's error allowance: every column whose
  * f16 score is within eps of the row's best is re-ranked (eps <= 0 selects the provable
- * default 2^-7 + 2^-11).  Rows whose candidate list overflowed are finished by the exact kernel, so the
+ * default: 2^-9 + 2^-10 + 2^-16 for d_pad <= 4096, 2^-9 + d_pad * (2^-22 + 2^-28) for wider rows).
+ * Rows whose candidate list overflowed are finished by the exact kernel, so the
  * result never depends on the screen's precision.  q_* may equal x_* (FINCH self-search). */
 int slic_nn_top1(const void* q_unit_dev, const uint16_t* q_f16_dev, int64_t nq,
                  const void* x_unit_dev, const uint16_t* x_f16_dev, int64_t n,

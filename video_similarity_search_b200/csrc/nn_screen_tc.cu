@@ -123,6 +123,19 @@ constexpr int TC_THREADS_SYM = TC_THREADS + 32;
 // <= 2^-11.  eps must be >= twice the worst-case |screened - exact|: 2 * (2^-10 + 2^-11 + 2^-18) < 2^-9 + 2^-10 + 2^-16.
 // (The first version screened in bfloat16 with eps = 2^-7 + 2^-11: 2.8 x as wide a band, several times the candidates.)
 constexpr float TC_DEFAULT_EPS = 0.001953125f + 0.0009765625f + 0.0000152587890625f;
+// Wider rows (d_pad > 4096).  For any width the worst case is, term by term:
+//   rounding of the normal components      (2^-10 + 2^-22) * sum|a_k b_k| <= 2^-10 + 2^-22
+//   subnormal components                   2^-25 * (sum|a_k| + sum|b_k|) <= 2^-24 * sqrt(d_pad)   (Cauchy-Schwarz)
+//   float32 accumulation                   d_pad * 2^-23 * max|partial sum| <= d_pad * 2^-23 * (1 + 2^-9)
+// Twice that is 2^-9 + d_pad * 2^-22 + (2^-21 + 2^-23 * sqrt(d_pad) + d_pad * 2^-31), and the bracket is <= d_pad * 2^-28
+// for every d_pad >= 4096 (at 4096: 1.00e-5 <= 1.53e-5, and the right side grows faster).  So
+//   eps(d_pad) = 2^-9 + d_pad * (2^-22 + 2^-28)
+// covers the bound at every width above 4096, grows with the accumulation term and equals TC_DEFAULT_EPS at 4096, where
+// the two rules meet.  Up to 4096 the constant is kept as it is.
+static float screen_default_eps(int d_pad) {
+    if (d_pad <= 4096) return TC_DEFAULT_EPS;
+    return (float)(0.001953125 + (double)d_pad * (0x1p-22 + 0x1p-28));
+}
 constexpr int TC_TOPK_MAX = 64;  // the top-k variant's per-row score histogram has saturating 8-bit counts: k must stay well below 255
 constexpr int TC_HIST_BINS = 128;
 constexpr int TC_HIST_STRIDE = 2 * TC_BM;   // one histogram per (row, column half)
@@ -2481,17 +2494,18 @@ int nn_top1_f32_gated(const float* q_unit, const uint16_t* q_f16, int64_t nq, co
                       const uint16_t* x_f16, int64_t n, int d, int d_pad, int64_t self_offset, float eps, int* idx_out,
                       float* dist_out, int* stats_out, const GateSpec* gate, AfterScreenFn after, void* after_ctx,
                       cudaStream_t st, int* stats_ext) {
-    if (eps <= 0.f) eps = TC_DEFAULT_EPS;
+    if (eps <= 0.f) eps = screen_default_eps(d_pad);
     return nn_top1_impl<float>(q_unit, q_f16, nq, x_unit, x_f16, n, d, d_pad, self_offset, eps, idx_out, dist_out,
                                stats_out, st, gate, after, after_ctx, stats_ext);
 }
 
 int nn_top1_self_async(const void* unit, const uint16_t* ub, int64_t n, int d, int d_pad, int dtype, int* idx_out,
                        void* dist_out, int* stats_ext, cudaStream_t st) {
+    const float eps = screen_default_eps(d_pad);
     if (dtype == SLIC_F32)
-        return nn_top1_impl<float>((const float*)unit, ub, n, (const float*)unit, ub, n, d, d_pad, 0, TC_DEFAULT_EPS,
-                                   idx_out, (float*)dist_out, nullptr, st, nullptr, nullptr, nullptr, stats_ext);
-    return nn_top1_impl<double>((const double*)unit, ub, n, (const double*)unit, ub, n, d, d_pad, 0, TC_DEFAULT_EPS, idx_out,
+        return nn_top1_impl<float>((const float*)unit, ub, n, (const float*)unit, ub, n, d, d_pad, 0, eps, idx_out,
+                                   (float*)dist_out, nullptr, st, nullptr, nullptr, nullptr, stats_ext);
+    return nn_top1_impl<double>((const double*)unit, ub, n, (const double*)unit, ub, n, d, d_pad, 0, eps, idx_out,
                                 (double*)dist_out, nullptr, st, nullptr, nullptr, nullptr, stats_ext);
 }
 
@@ -2503,8 +2517,8 @@ int nn_top1_sym_fused(const float* unit, const uint16_t* ub, int64_t n, int d, i
         return SLIC_ERR_UNSUPPORTED;
     }
     bool overflowed = false;
-    return nn_top1_sym_impl<float>(unit, ub, n, d, d_pad, TC_DEFAULT_EPS, idx_out, dist_out, nullptr, st, part, parts, nullptr,
-                                   nullptr, nullptr, &overflowed, SYM_FUSED, nullptr, nullptr, stats_dev, peers,
+    return nn_top1_sym_impl<float>(unit, ub, n, d, d_pad, screen_default_eps(d_pad), idx_out, dist_out, nullptr, st, part,
+                                   parts, nullptr, nullptr, nullptr, &overflowed, SYM_FUSED, nullptr, nullptr, stats_dev, peers,
                                    before_screen, before_ctx);
 }
 
@@ -2522,7 +2536,7 @@ int slic_nn_top1(const void* q_unit_dev, const uint16_t* q_f16_dev, int64_t nq, 
     SLIC_REQUIRE((reinterpret_cast<uintptr_t>(q_f16_dev) & 15) == 0 && (reinterpret_cast<uintptr_t>(x_f16_dev) & 15) == 0,
                  "nn_top1: f16 matrices must be 16-byte aligned");
     SLIC_PROPAGATE(slic_require_device());
-    if (eps <= 0.f) eps = slic::TC_DEFAULT_EPS;
+    if (eps <= 0.f) eps = slic::screen_default_eps(d_pad);
     cudaStream_t st = slic::as_stream(stream);
     if (dtype == SLIC_F32)
         return slic::nn_top1_impl<float>((const float*)q_unit_dev, q_f16_dev, nq, (const float*)x_unit_dev, x_f16_dev,
@@ -2547,7 +2561,7 @@ int slic_sym_row_bests(const float* unit_dev, const uint16_t* f16_dev, int64_t n
         return SLIC_ERR_UNSUPPORTED;
     }
     bool overflowed = false;
-    return nn_top1_sym_impl<float>(unit_dev, f16_dev, n, d, d_pad, TC_DEFAULT_EPS, nullptr, nullptr, nullptr,
+    return nn_top1_sym_impl<float>(unit_dev, f16_dev, n, d, d_pad, screen_default_eps(d_pad), nullptr, nullptr, nullptr,
                                    as_stream(stream), part, parts, nullptr, nullptr, nullptr, &overflowed, SYM_BESTS, nullptr,
                                    bests_out_dev);
 }
@@ -2567,7 +2581,7 @@ int slic_nn_top1_sym_part(const float* unit_dev, const uint16_t* f16_dev, int64_
                   (long long)SYM_MIN_ROWS_FWD);
         return SLIC_ERR_UNSUPPORTED;
     }
-    if (eps <= 0.f) eps = TC_DEFAULT_EPS;
+    if (eps <= 0.f) eps = screen_default_eps(d_pad);
     cudaStream_t st = as_stream(stream);
     Scratch idx, dist;
     SLIC_CUDA_OK(idx.alloc((size_t)n * sizeof(int), st));
@@ -2645,7 +2659,7 @@ int slic_topk_cosine_tc(const void* q_unit_dev, const uint16_t* q_f16_dev, int64
                  "topk_cosine_tc: f16 matrices must be 16-byte aligned");
     if (nq == 0) return SLIC_OK;
     SLIC_PROPAGATE(slic_require_device());
-    if (eps <= 0.f) eps = slic::TC_DEFAULT_EPS;
+    if (eps <= 0.f) eps = slic::screen_default_eps(d_pad);
     cudaStream_t st = slic::as_stream(stream);
     if (dtype == SLIC_F32)
         return slic::topk_tc_impl<float>((const float*)q_unit_dev, q_f16_dev, nq, (const float*)x_unit_dev, x_f16_dev,
@@ -2713,7 +2727,7 @@ int slic_screen_scores_debug(const uint16_t* q_f16_dev, int64_t nq, const uint16
     SLIC_CUDA_OK(cf.alloc(slots * sizeof(int), st));
     SLIC_CUDA_OK(err.alloc(sizeof(int), st));
     SLIC_CUDA_OK(cudaMemsetAsync(err.ptr, 0, sizeof(int), st));
-    SLIC_PROPAGATE(launch_screen(q_f16_dev, nq, x_f16_dev, n, d_pad, -1, TC_DEFAULT_EPS, TC_CAP, pl, ci.as<int>(),
+    SLIC_PROPAGATE(launch_screen(q_f16_dev, nq, x_f16_dev, n, d_pad, -1, screen_default_eps(d_pad), TC_CAP, pl, ci.as<int>(),
                                  cs.as<float>(), cc.as<int>(), cf.as<int>(), out_dev, err.as<int>(), st));
     int host_err = 0;
     SLIC_CUDA_OK(cudaMemcpyAsync(&host_err, err.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
